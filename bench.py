@@ -176,8 +176,8 @@ def build_product(device, aux, hybrid=False, workload="c3"):
     import preprocess_helpers as pre
     from pipeline import FusionPipeline
 
+    torch.manual_seed(0)  # before make_params: the c4 / resnet backbones draw their weights there
     params, backbones = make_params(workload, hybrid)
-    torch.manual_seed(0)
     mods = [mm.initialize_model(mm.ModelMaskHeadBackbone("dwi", params, backbones["dwi"]), True),
             mm.initialize_model(mm.ModelMaskHeadBackbone("dce", params, backbones["dce"]), True),
             mm.initialize_model(mm.FusionModel(params), True)]
@@ -200,6 +200,26 @@ def build_product(device, aux, hybrid=False, workload="c3"):
     pipe = FusionPipeline(mods[0], mods[1], mods[2], nyul, aux_mode=aux,
                           input_size=224 if workload != "c3" else None).eval()
     return params, pipe, cpu_state, nyul
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: {name: tensor} -> directory/<name>.npy, float32.  When the arrays exceed DUMP_BYTES together,
+    every one is cut to the same fixed stride of its flattened elements, so repeated runs store the same sample."""
+    import numpy as np
+
+    arrays = {k: v.detach().float() for k, v in arrays.items()}
+    total = sum(v.numel() for v in arrays.values()) * 4
+    stride = -(-total // DUMP_BYTES)
+    os.makedirs(directory, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), (v if stride == 1 else v.reshape(-1)[::stride]).cpu().numpy())
+
+
+def flat_parameters(params):
+    return torch.cat([q.detach().float().reshape(-1) for q in params])
 
 
 # --------------------------------------------------------------------- CPU baseline ----
@@ -360,6 +380,9 @@ def train_arm(args):
         barrier()
         torch.cuda.nvtx.range_pop()
     launches = nat.LAUNCH_COUNT - launches0
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1),
+                                         "fusion_parameters": flat_parameters(pipe.fusion_model.parameters())})
     ms = e0.elapsed_time(e1)
     # end to end: pinned host batch (inputs + labels) uploaded every step, the loss read back every step
     dwi_p, dce_p, lab_p, msk_p = dwi_h.pin_memory(), dce_h.pin_memory(), lab_h.pin_memory(), msk_h.pin_memory()
@@ -566,6 +589,8 @@ def train_full_arm(args):
         barrier()
         torch.cuda.nvtx.range_pop()
     launches = nat.LAUNCH_COUNT - launches0
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1), "trained_parameters": flat_parameters(trainer.params)})
     ms = e0.elapsed_time(e1)
     # end to end: pinned host batch uploaded every step (copy stream, overlapped with the previous step), loss read back
     host_batch = tuple(t.pin_memory() for t in (dwi_h, dce_h, lab_h, msk_h))
@@ -705,6 +730,8 @@ def c1_arm(args):
         torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
     launches = nat.LAUNCH_COUNT - l0
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1), "dwi_parameters": flat_parameters(model.parameters())})
     m_h, l_h = masks.pin_memory(), labels.pin_memory()
     e0.record()
     for _ in range(args.steps):
@@ -821,7 +848,17 @@ def main():
                          "the reference's default test_mode.  Not the headline workload.")
     ap.add_argument("--hybrid", action="store_true",
                     help="encoders with the in-house TransformerStage instead of block3 (not the headline workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32, at most "
+                         "64 MB): the fusion logits of every case, gathered over the ranks (fusion_probabilities in the "
+                         "multi-pass predict modes); for c5 / c1 the loss and the parameters after the update.  Inputs "
+                         "and weights are seeded, so two builds can be compared output for output; repeated runs of one "
+                         "build are close, not bit-identical (the encoders' channel sums are float atomics)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 path")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     if args.workload == "c1":
@@ -914,11 +951,15 @@ def main():
         torch.cuda.nvtx.range_push("timed")  # ncu --nvtx --nvtx-include "timed/" captures exactly these steps
         e0.record()
         per_step = [step() for _ in range(args.steps)]
-        gather(per_step)
+        gathered = gather(per_step)
         e1.record()
         barrier()
         torch.cuda.nvtx.range_pop()
     launches = nat.LAUNCH_COUNT - launches0
+    if args.dump_outputs is not None and rank == 0:
+        last = per_step[-1] if gathered is None else gathered[:, -1].reshape(-1, per_step[-1].shape[-1])
+        # the multi-pass prediction modes return the mean softmax over their passes, not logits
+        dump_outputs(args.dump_outputs, {"fusion_logits" if args.predict_mode == "normal" else "fusion_probabilities": last})
     ms = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms], device=device)

@@ -51,7 +51,8 @@ with open(os.path.join(out_dir, f"{tag}_sass_summary.md"), "w") as f:
             "count and the count of the mnemonics that identify the Blackwell-native paths (UTCHMMA = tcgen05.mma, "
             "LDTM = tcgen05.ld, UTMALDG/UTMASTG = TMA load/store, SYNCS = mbarrier, FFMA2/FMUL2/FADD2 = packed fp32x2; "
             "LD/ST = generic-space accesses, which the hot kernels should not have).  No HMMA (legacy mma.sync) anywhere.  "
-            f"The complete listing of every kernel is `{tag}_all_kernels.sass.gz`; six representative kernels are also "
+            f"The tool writes the complete listing of every kernel to `{tag}_all_kernels.sass.gz` (a build product, not "
+            "kept in git); six representative kernels are "
             "stored uncompressed next to this file.\n\n")
     f.write("| kernel | instr | " + " | ".join(COLS) + " |\n|---|---|" + "---|" * len(COLS) + "\n")
     for d, n, ops, _ in rows:
