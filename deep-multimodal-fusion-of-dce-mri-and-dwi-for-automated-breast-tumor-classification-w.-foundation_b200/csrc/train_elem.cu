@@ -681,17 +681,21 @@ convc1_fwd_kernel(const __nv_bfloat16* __restrict__ x, int ldx, int H, int W, in
             for (int t = 0; t < TAPS; ++t) wr[k][t] = __ldg(w + (c0 + k) * TAPS + t);
         }
         constexpr int NP = 4;  // pixels per trip: their loads are issued together (the loop is latency bound otherwise)
-        for (int pix0 = slot; pix0 < npix; pix0 += NP * nslots) {
+        // The trip / break conditions use the warp's first pixel slot so that every lane reaches the full-warp shuffles
+        // below; a lane past the last pixel reduces zeros and stores nothing.
+        const int wslot = slot - grp;
+        for (int w0 = wslot; w0 < npix; w0 += NP * nslots) {
             uint4 q[NP];
 #pragma unroll
             for (int h = 0; h < NP; ++h) {
-                const int pix = pix0 + h * nslots;
-                if (pix < npix) q[h] = __ldg(reinterpret_cast<const uint4*>(x + (static_cast<long long>(b) * npix + pix) * ldx + c0));
+                const int pix = w0 + grp + h * nslots;
+                q[h] = pix < npix ? __ldg(reinterpret_cast<const uint4*>(x + (static_cast<long long>(b) * npix + pix) * ldx + c0))
+                                  : make_uint4(0u, 0u, 0u, 0u);
             }
 #pragma unroll
             for (int h = 0; h < NP; ++h) {
-                const int pix = pix0 + h * nslots;
-                if (pix >= npix) break;
+                if (w0 + h * nslots >= npix) break;
+                const int pix = w0 + grp + h * nslots;
                 float acc[TAPS];
 #pragma unroll
                 for (int t = 0; t < TAPS; ++t) acc[t] = 0.f;
@@ -708,7 +712,7 @@ convc1_fwd_kernel(const __nv_bfloat16* __restrict__ x, int ldx, int H, int W, in
                     for (int o = gl >> 1; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
                     acc[t] = v;
                 }
-                if (sub == 0) {  // (C > 256: the same lane revisits the pixel with the next 256 channels)
+                if (sub == 0 && pix < npix) {  // (C > 256: the same lane revisits the pixel with the next 256 channels)
 #pragma unroll
                     for (int t = 0; t < TAPS; ++t) s_d[pix * TAPS + t] = (c0 < 256 ? 0.f : s_d[pix * TAPS + t]) + acc[t];
                 }
@@ -887,7 +891,7 @@ lift_bwd_kernel(const __nv_bfloat16* __restrict__ dz, const float* __restrict__ 
 
 // --------------------------------------------------------------------------- mask-guided modulation backward -----
 // forward: y = f * (1 + gamma * A[b,p]).   backward (one warp per pixel):
-//   df[b,p,c] (+)= dy * (1 + gamma A);  dA[b,p] = gamma * sum_c dy * f;  dgamma += sum dy * f * A
+//   df[b,p,c] = dy * (1 + gamma A);  dA[b,p] = gamma * sum_c dy * f;  dgamma += sum dy * f * A
 __global__ void __launch_bounds__(kTeThreads)
 modulate_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, const __nv_bfloat16* __restrict__ f, int ldf,
                     const float* __restrict__ A, const float* __restrict__ gamma, long long P, int C,
@@ -926,7 +930,7 @@ modulate_bwd_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, const __nv_b
 // ------------------------------------------------------------------- mask attention (1 -> 16 -> 1) backward ------
 // forward per case: u[p,k] = wa[k] m[p];  GroupNorm(1, K) over all (p, k);  g = gelu(gn);  s[p] = sum_k wb[k] g[p,k] + bb;
 // A = clamp(sigmoid(s), 1e-4, 1 - 1e-4).  One CTA per case; K <= 32; the map is recomputed, nothing was saved.
-// Outputs: dm[b,p] (+= if accumulate), dwa[K], dgnw[K], dgnb[K], dwb[K], dbb accumulated atomically.
+// Outputs: dm[b,p] overwritten; dwa[K], dgnw[K], dgnb[K], dwb[K], dbb accumulated atomically.
 __global__ void __launch_bounds__(kTeThreads)
 mask_attn_bwd_kernel(const float* __restrict__ mask, const float* __restrict__ dA, int npix, int K,
                      const float* __restrict__ wa, const float* __restrict__ gnw, const float* __restrict__ gnb,
@@ -1841,8 +1845,11 @@ extern "C" int b200_mask_attn_bwd(const float* mask, const float* dA, int B, int
 
 extern "C" int b200_stem_bwd(const float* x, int B, int C, int H, int W, int stride, const float* gate, const void* dz,
                              int N, const float* wcat, float* dwcat, float* dgate, void* stream) {
-    if (x == nullptr || dz == nullptr || wcat == nullptr || dwcat == nullptr || C > 32 || N > kTeThreads || N % 8 != 0 || B <= 0)
+    if (x == nullptr || dz == nullptr || wcat == nullptr || dwcat == nullptr || C <= 0 || C > 32 || N > kTeThreads || N % 8 != 0 ||
+        B <= 0)
         return -1;
+    // the forward (b200_stem_ex) takes every stride-th pixel of an H x W plane that the stride divides
+    if (stride < 1 || H % stride != 0 || W % stride != 0) return -1;
     const int CP = C <= 8 ? 8 : (C <= 16 ? 16 : 32);
     const size_t smem = (static_cast<size_t>(N) * CP + static_cast<size_t>(kTeThreads) * CP + CP) * sizeof(float);
     auto go = [&](auto kern) -> int {

@@ -53,6 +53,63 @@ def test_invalid_arguments_are_rejected_without_a_gpu():
     assert lib.b200_stem(None, 1, 64, 8, 8, 2, None, None, None, None, None, 0, None, None, None, 8, 8, None, None, None, None) < 0
 
 
+def test_training_kernels_reject_out_of_range_arguments_without_a_gpu():
+    """csrc/train_elem.cu: every documented limit returns < 0 before anything is launched (the pointers are never read:
+    any non-NULL value stands for a buffer)."""
+    import b200_native as nat
+
+    lib, p = nat.lib(), 16
+    assert lib.b200_bn_stats(p, 100, 12, 16, p, p, None) == -1                           # C % 8
+    assert lib.b200_bn_stats(p, 100, 2056, 2056, p, p, None) == -1                       # C > 2048
+    assert lib.b200_bn_finalize(p, p, 8, 0.0, 1e-5, 0.1, None, None, p, p, None) == -1   # count <= 0
+    bn = (p, 8, None, 8, p, p, p, p)
+    assert lib.b200_bn_act_fwd(p, 16, None, 16, p, p, p, p, 1, 0.0, 0, 10, 12, p, 16, None) == -1   # C % 8
+    assert lib.b200_bn_act_fwd(*bn, 3, 0.0, 0, 10, 8, p, 8, None) == -2                  # act
+    assert lib.b200_bn_act_fwd(*bn, 1, 1.0, 0, 10, 8, p, 8, None) == -2                  # drop_p >= 1
+    assert lib.b200_bn_act_fwd(p, 1032, None, 8, p, p, p, p, 1, 0.0, 0, 10, 1032, p, 1032, None) == -3  # C > 1024
+    assert lib.b200_bn_act_bwd(p, 1032, None, 8, p, p, p, p, 1, 0.0, 0, 10, 1032, p, 1032, 1, p, p, 1032, None, 0, p, p,
+                               None) == -3
+    assert lib.b200_bn_act_bwd(*bn, 1, 0.0, 0, 10, 8, p, 8, 1, p, None, 8, None, 0, p, p, None) == -5  # pass 2 needs dz
+    assert lib.b200_bn_act_bwd(*bn, 1, 0.0, 0, 10, 8, p, 8, 1, None, p, 8, None, 0, p, p, None) == -4  # no scratch
+    assert lib.b200_map_dot(p, 2056, None, 0, 2, 10, 2056, p, None) == -1                # C > 2048
+    assert lib.b200_map_scale_add(p, 16, p, p, 2, 10, 12, p, 16, 0, None) == -1          # C % 8
+    assert lib.b200_map_axpby(p, 16, 1.0, None, 0, 0.0, 10, 12, p, 16, None) == -1
+    assert lib.b200_map_sumsq(p, 8, 0, 8, p, None) == -1                                 # R <= 0
+    assert lib.b200_se_fwd(p, 2, 64, 0, 49, p, p, p, p, p, p, None) == -1                # M <= 0
+    assert lib.b200_se_bwd(p, p, p, p, p, p, 2, 6200, 1, p, p, p, p, None) == -2         # shared memory > 48 KB
+    for C, taps, H, W in ((24, 9, 8, 8), (288, 1, 8, 8), (64, 4, 8, 8), (64, 9, 200, 200)):  # convc1_shape_ok
+        assert lib.b200_convc1_fwd(p, C, 2, H, W, C, taps, p, p, p, None) == -1
+        assert lib.b200_convc1_bwd(p, C, p, 2, H, W, C, taps, p, p, C, 0, p, p, None) == -1
+    assert lib.b200_convc1_bwd(p, 2048, p, 2, 250, 200, 2048, 1, p, p, 2048, 0, p, p, None) == -2  # dout + dw > 200 KB
+    assert lib.b200_lift_fwd(p, 10, 12, p, p, None) == -1                                # N % 8
+    assert lib.b200_lift_bwd(p, p, 10, 136, p, p, p, None) == -1                         # N > 128
+    assert lib.b200_modulate_bwd(p, 16, p, 16, p, p, 10, 12, p, 16, p, p, None) == -1    # C % 8
+    assert lib.b200_mask_attn_bwd(p, p, 2, 256, 33, p, p, p, p, p, 1e-5, p, p, p, p, p, p, None) == -1  # K > 32
+    stem = (p, 2, 3, 16, 16)
+    assert lib.b200_stem_bwd(*stem, 2, p, p, 264, p, p, p, None) == -1                   # N > 256
+    assert lib.b200_stem_bwd(p, 2, 33, 16, 16, 2, p, p, 64, p, p, p, None) == -1         # C > 32
+    assert lib.b200_stem_bwd(p, 2, 3, 15, 16, 2, p, p, 64, p, p, p, None) == -1          # H % stride (as b200_stem_ex)
+    assert lib.b200_stem_bwd(p, 2, 3, 16, 17, 2, p, p, 64, p, p, p, None) == -1          # W % stride
+    assert lib.b200_stem_bwd(*stem, 0, p, p, 64, p, p, p, None) == -1                    # stride < 1
+    assert lib.b200_cls_head_bwd(p, p, p, 2, 64, 17, 1, p, p, p, None) == -1             # K > 16
+    assert lib.b200_focal_loss(p, p, 2, 17, 0.1, 2.0, None, 1.0, p, p, None) == -1       # K > 16
+    assert lib.b200_dice_loss(p, p, 2, 0, 1.0, 1.0, p, p, None) == -1                    # n <= 0
+    assert lib.b200_recon_loss(p, 2, 128, 65, p, 1, None, 0, 256, 130, 1e-3, 1.0, p, p, None) == -1  # h w > 8192
+    assert lib.b200_recon_loss(p, 2, 16, 16, p, 1, None, 2, 64, 64, 1e-3, 1.0, p, p, None) == -1    # x2 NULL, C2 > 0
+    assert lib.b200_mimic_loss(p, p, 2, 12, 1.0, p, p, None) == -1                       # n % 8
+    assert lib.b200_gating_fwd(p, p, 0, 64, 49, None, None, 0, p, p, p, p, None) == -1   # B <= 0
+    assert lib.b200_gating_bwd(p, p, p, 2, 64, 128, 0, p, p, p, p, None) == -1           # npix <= 0
+    assert lib.b200_fused_pool(p, p, 2, 64, 49, None, None, None, 0, p, None) == -1      # alpha NULL
+    mix = (p, p, p, p, 2, 14, 14)
+    assert lib.b200_fusion_mix_bwd(*mix, 12, 7, 7, p, p, None, None, None, None, None, None, 0, None) == -1  # C % 8
+    assert lib.b200_fusion_mix_bwd(*mix, 512, 7, 7, p, p, None, None, None, None, None, None, 0, None) == -3  # smem
+    assert lib.b200_fusion_mix_bwd(*mix, 64, 3, 7, None, None, p, p, p, p, p, p, 1, None) == -4  # dtok, H % Hp
+    assert lib.b200_mimic_pairs(p, 3, 49, 64, 1.0, p, p, None) == -1                     # B < 4
+    assert lib.b200_up2_bwd(p, 2, 7, 7, 12, p, None) == -1                               # C % 8
+    assert lib.b200_row_bcast(p, 1, 1.0, 2, 0, p, None) == -1                            # n <= 0
+    assert lib.b200_vec_axpby(p, 1.0, 0.0, 0, p, None) == -1                             # n <= 0
+
+
 def test_missing_library_fails_loudly(monkeypatch):
     import b200_native as nat
 
