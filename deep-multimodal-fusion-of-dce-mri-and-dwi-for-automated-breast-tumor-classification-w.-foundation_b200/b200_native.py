@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # csrc/build.sh links the library at <repo>/lib/libb200fusion.so: a short path without the dots and dashes of the
 # package directory name, which is the path string dlopen sees.
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb200fusion.so")
-ABI_VERSION = 21
+ABI_VERSION = 22
 
 _lib = None
 
@@ -98,6 +98,7 @@ SIGNATURES = {
     "b200_conv_gemm_mc": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _P, _I, _P, _I, _I, _P, _I, _F, _P, _I, _I, _I,
                           _I, _I, _I, _I, _I, _F, C.c_ulonglong, _I, _P],
     "b200_attention": [_P, _I, _P, _I, _I, _I, _I, _I, _F, _P],
+    "b200_attention_mc": [_P, _I, _P, _I, _I, _I, _I, _I, _F, _F, C.c_ulonglong, _P],
     "b200_resize_bilinear_c1": [_P, _I, _I, _I, _P, _I, _I, _P],
     "b200_resize_aa_c1": [_P, _I, _I, _I, _P, _I, _I, _P],
     "b200_mask_attention": [_P, _I, _I, _I, _P, _P, _P, _P, _P, _F, _P, _P],
@@ -108,6 +109,7 @@ SIGNATURES = {
     "b200_vit_tokens": [_P, _P, _P, _I, _I, _I, _P, _P],
     "b200_vit_feature": [_P, _I, _I, _I, _P, _I, _P],
     "b200_linear": [_P, _LL, _I, _P, _I, _P, _P, _P, _I, _I, _I, _P, _I, _P],
+    "b200_linear_mc": [_P, _LL, _I, _P, _I, _P, _P, _P, _I, _I, _I, _P, _I, _F, C.c_ulonglong, _P],
     "b200_dwi_normalize": [_P, _P, _I, _I, _I, _I, _F, _F, _P, _P],
     "b200_dwi_normalize_ex": [_P, _P, _I, _I, _I, _I, _F, _F, _P, _P, _P],
     "b200_nyul_transform_ex2": [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P],
@@ -352,15 +354,21 @@ def layernorm(x, w, b, eps, out=None, out_dtype=torch.bfloat16):
     return out
 
 
-def linear_f32(x2d, w, *, scale=None, bias=None, res=None, res_mode=0, act=0, out=None, out_dtype=torch.bfloat16):
-    """x2d [M,K] bf16, w [N,K] bf16; residual / output may be fp32 [M,N] (the transformer residual stream)."""
+def linear_f32(x2d, w, *, scale=None, bias=None, res=None, res_mode=0, act=0, out=None, out_dtype=torch.bfloat16,
+               dropout=None):
+    """x2d [M,K] bf16, w [N,K] bf16; residual / output may be fp32 [M,N] (the transformer residual stream).
+    dropout = (p, seed): MC dropout before the residual add, out = res + drop(act(x w^T * scale + bias))
+    (b200_linear_mc)."""
     M, K = x2d.shape
     N = w.shape[0]
     if out is None:
         out = torch.empty((M, N), dtype=out_dtype, device=x2d.device)
-    _call("b200_linear", (M, K, N), _ptr(x2d), M, K, _ptr(w), N, _ptr(scale), _ptr(bias), _ptr(res),
-          int(res is not None and res.dtype == torch.float32), res_mode, act, _ptr(out),
-          int(out.dtype == torch.float32), _stream())
+    args = (_ptr(x2d), M, K, _ptr(w), N, _ptr(scale), _ptr(bias), _ptr(res),
+            int(res is not None and res.dtype == torch.float32), res_mode, act, _ptr(out), int(out.dtype == torch.float32))
+    if dropout is not None:
+        _call("b200_linear_mc", (M, K, N), *args, float(dropout[0]), int(dropout[1]) & 0xFFFFFFFFFFFFFFFF, _stream())
+    else:
+        _call("b200_linear", (M, K, N), *args, _stream())
     return out
 
 
@@ -427,12 +435,14 @@ def tapsum(d, bias, out):
     return out
 
 
-def linear(x2d, w, *, scale=None, bias=None, res=None, res_mode=0, act=0, out=None):
-    """Plain GEMM: x2d [M,K] bf16, w [N,K] bf16 -> [M,N] bf16 with the same fused epilogue."""
+def linear(x2d, w, *, scale=None, bias=None, res=None, res_mode=0, act=0, out=None, dropout=None):
+    """Plain GEMM: x2d [M,K] bf16, w [N,K] bf16 -> [M,N] bf16 with the same fused epilogue.  dropout = (p, seed): MC
+    dropout after the activation (and after a residual), element (row, col) decided by Philox(seed; row * N + col)."""
     M, K = x2d.shape
     y = conv_gemm(x2d.view(1, 1, M, K), w, taps=1, scale=scale, bias=bias,
                   res=None if res is None else res.view(1, 1, M, -1), res_mode=res_mode, act=act,
-                  out=None if out is None else out.view(1, 1, M, -1))
+                  out=None if out is None else out.view(1, 1, M, -1),
+                  dropout=None if dropout is None else (dropout[0], dropout[1], 1))
     return y.view(M, -1)
 
 
@@ -453,12 +463,18 @@ def nyul_transform(x, out, C_, n, avg_landmarks, standard_scale, prev_index, gam
     return out
 
 
-def attention(qkv, out, B, N, heads, dh, scale=None):
+def attention(qkv, out, B, N, heads, dh, scale=None, dropout=None):
     """Fused softmax(q k^T * scale) v over the packed qkv rows [B*N, 3*heads*dh] bf16 -> out [B*N, heads*dh] bf16
-    (b200_attention; transformer_model.py:101-112)."""
+    (b200_attention; transformer_model.py:101-112).  dropout = (p, seed): attention dropout on the probabilities
+    (b200_attention_mc)."""
     assert qkv.dtype == torch.bfloat16 and out.dtype == torch.bfloat16 and qkv.stride(-1) == 1 and out.stride(-1) == 1
-    _call("b200_attention", (B, N, heads, dh), _ptr(qkv), qkv.stride(0), _ptr(out), out.stride(0), B, N, heads, dh,
-          float(dh ** -0.5 if scale is None else scale), _stream())
+    args = (_ptr(qkv), qkv.stride(0), _ptr(out), out.stride(0), B, N, heads, dh,
+            float(dh ** -0.5 if scale is None else scale))
+    if dropout is not None:
+        _call("b200_attention_mc", (B, N, heads, dh), *args, float(dropout[0]), int(dropout[1]) & 0xFFFFFFFFFFFFFFFF,
+              _stream())
+    else:
+        _call("b200_attention", (B, N, heads, dh), *args, _stream())
     return out
 
 

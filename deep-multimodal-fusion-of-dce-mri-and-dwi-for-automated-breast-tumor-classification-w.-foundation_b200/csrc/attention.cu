@@ -49,6 +49,11 @@ struct AttnParams {
     int out_ld;
     float scale_log2;  // scale * log2(e)
     __nv_bfloat16* out;
+    // attention dropout (attn_fused_kernel<DH, true> only): probability (case b, head h, query row, key j) is dropped
+    // when word j % 4 of Philox4x32-7(seed; ((b * heads + h) * N + row) * 64 + j / 4) < drop_thresh
+    unsigned int drop_thresh;
+    float drop_scale;  // 1 / (1 - p), folded into the row's 1 / sum
+    unsigned int drop_seed_lo, drop_seed_hi;
 };
 
 __device__ __forceinline__ uint64_t at_desc_mn_sw128(uint32_t smem_addr, uint32_t lbo_bytes) {
@@ -63,11 +68,15 @@ __device__ __forceinline__ uint64_t at_desc_mn_sw128(uint32_t smem_addr, uint32_
 
 // 32 scores of one row -> probabilities (unnormalised), stored as bf16 in the row's four 16-byte pieces of the
 // swizzled [128 x 128 B] slice; returns their fp32 sum.  MASK: columns >= valid are past the case's last key -> 0.
-template <bool MASK>
+// DROP: the sum is that of the undropped probabilities (the softmax denominator); dropped ones are stored as 0.
+// `ctr` is the Philox counter of the chunk's first four keys (see AttnParams).
+template <bool MASK, bool DROP>
 __device__ __forceinline__ float softmax_chunk(const uint32_t (&v)[32], float scale_log2, float mneg, int valid,
-                                               uint8_t* dst, int j0, int swz) {
+                                               uint8_t* dst, int j0, int swz, const AttnParams& p,
+                                               unsigned long long ctr) {
     uint32_t pk[16];
     float s4[4] = {0.f, 0.f, 0.f, 0.f};
+    uint4 rnd = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
     for (int i = 0; i < 32; i += 2) {
         float e0 = ex2_approx(fmaf(__uint_as_float(v[i]), scale_log2, mneg));
@@ -77,6 +86,12 @@ __device__ __forceinline__ float softmax_chunk(const uint32_t (&v)[32], float sc
             if (i + 1 >= valid) e1 = 0.f;
         }
         s4[(i >> 1) & 3] += e0 + e1;
+        if (DROP) {
+            if ((i & 3) == 0) rnd = philox4x32_7(ctr + (i >> 2), p.drop_seed_lo, p.drop_seed_hi);
+            const uint32_t r0 = (i & 3) == 0 ? rnd.x : rnd.z, r1 = (i & 3) == 0 ? rnd.y : rnd.w;
+            if (r0 < p.drop_thresh) e0 = 0.f;
+            if (r1 < p.drop_thresh) e1 = 0.f;
+        }
         const __nv_bfloat162 t = __floats2bfloat162_rn(e0, e1);
         pk[i >> 1] = *reinterpret_cast<const uint32_t*>(&t);
     }
@@ -88,7 +103,8 @@ __device__ __forceinline__ float softmax_chunk(const uint32_t (&v)[32], float sc
 }
 
 // One query row per thread: scores S[row, 0:N] in TMEM (lane = row) -> unnormalised probabilities as bf16 into the
-// swizzled K-major slices of `s_p`; returns 1 / (fp32 row sum).
+// swizzled K-major slices of `s_p`; returns 1 / (fp32 row sum), times 1 / (1 - p) with DROP.  `ctr` = Philox counter
+// of the row's keys 0-3 (DROP only).
 //
 // Reading the scores back out of TMEM (64 B/clk per SM) is what bounds this kernel, so the common case reads them
 // ONCE: the reference point of the exponent is the max of the row's first 32 scores, not the row max.  Softmax is
@@ -96,7 +112,9 @@ __device__ __forceinline__ float softmax_chunk(const uint32_t (&v)[32], float sc
 // precision at any exponent); the true max is >= the reference, so nothing underflows, and overflow shows up as a
 // row sum that is not < 1e30 - any such row (scores rising by more than ~100 * ln 2 past the first chunk; not seen
 // on trained or random weights) sends its warp through the classic two-pass softmax instead.
-__device__ __forceinline__ float softmax_rows(uint32_t taddr, uint8_t* s_p, int r, const AttnParams& p) {
+template <bool DROP>
+__device__ __forceinline__ float softmax_rows(uint32_t taddr, uint8_t* s_p, int r, const AttnParams& p,
+                                              unsigned long long ctr) {
     const int swz = r & 7;
     float sum = 0.f;
     {
@@ -118,9 +136,9 @@ __device__ __forceinline__ float softmax_rows(uint32_t taddr, uint8_t* s_p, int 
             uint8_t* const dst = s_p + (c >> 1) * kAtQBox + r * 128;
             const int j0 = (c & 1) * 4;
             if (valid >= 32)
-                sum += softmax_chunk<false>(v, p.scale_log2, mneg, valid, dst, j0, swz);
+                sum += softmax_chunk<false, DROP>(v, p.scale_log2, mneg, valid, dst, j0, swz, p, ctr + c * 8);
             else
-                sum += softmax_chunk<true>(v, p.scale_log2, mneg, valid, dst, j0, swz);
+                sum += softmax_chunk<true, DROP>(v, p.scale_log2, mneg, valid, dst, j0, swz, p, ctr + c * 8);
         }
     }
     if (__any_sync(0xffffffffu, !(sum < 1.0e30f))) {  // overflow of the lazy reference somewhere in this warp
@@ -142,10 +160,10 @@ __device__ __forceinline__ float softmax_rows(uint32_t taddr, uint8_t* s_p, int 
             tmem_ld_wait32(v);
             const int valid = p.N - c * 32;
             uint8_t* const dst = s_p + (c >> 1) * kAtQBox + r * 128;
-            sum += softmax_chunk<true>(v, p.scale_log2, mneg, valid, dst, (c & 1) * 4, swz);
+            sum += softmax_chunk<true, DROP>(v, p.scale_log2, mneg, valid, dst, (c & 1) * 4, swz, p, ctr + c * 8);
         }
     }
-    return 1.0f / sum;
+    return (DROP ? p.drop_scale : 1.0f) / sum;
 }
 
 // O[row, 0:DH] in TMEM -> * inv_sum -> bf16 -> dst (the row's DH contiguous outputs); `store` = the row is a real query.
@@ -172,7 +190,7 @@ __device__ __forceinline__ void store_rows(uint32_t taddr, __nv_bfloat16* dst, b
     }
 }
 
-template <int DH>
+template <int DH, bool DROP>
 __global__ void __launch_bounds__(kAtThreads, DH == 64 ? 2 : 1)
 attn_fused_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV, const AttnParams p) {
     constexpr int KC = DH / 64;
@@ -276,7 +294,9 @@ attn_fused_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
             const bool warp_live = qt * 128 + warp * 32 < p.N;  // some row of this warp is a real query
             mbar_wait(bar_s, ph);
             tc_fence_after();
-            const float inv_sum = warp_live ? softmax_rows(taddr, s_p, r, p) : 0.f;
+            unsigned long long ctr = 0;
+            if (DROP) ctr = ((static_cast<unsigned long long>(b) * p.heads + h) * p.N + row) * 64;
+            const float inv_sum = warp_live ? softmax_rows<DROP>(taddr, s_p, r, p, ctr) : 0.f;
             fence_proxy_async_smem();  // P (generic-proxy stores) -> visible to the MMA's async-proxy reads
             tc_fence_before();
             mbar_arrive(bar_p);
@@ -327,7 +347,7 @@ static int at_encode_map(AtEncodeTiledFn enc, CUtensorMap* tm, const void* base,
     return r == CUDA_SUCCESS ? 0 : -300 - static_cast<int>(r);
 }
 
-template <int DH>
+template <int DH, bool DROP>
 static int at_launch(const CUtensorMap& tmQ, const CUtensorMap& tmKV, const AttnParams& p, int num_sms, cudaStream_t s) {
     constexpr int KC = DH / 64;
     constexpr int kQKBytes = KC * (kAtQBox + kAtKBox);
@@ -335,21 +355,19 @@ static int at_launch(const CUtensorMap& tmQ, const CUtensorMap& tmKV, const Attn
     constexpr int smem = kRegionA + KC * kAtKBox + 128 /*barriers*/ + 1024 /*alignment slack*/;
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(attn_fused_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(attn_fused_kernel<DH, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return static_cast<int>(e);
         configured = true;
     }
     int grid = num_sms * (DH == 64 ? 2 : 1);
     if (grid > p.n_items) grid = p.n_items;
-    attn_fused_kernel<DH><<<grid, kAtThreads, smem, s>>>(tmQ, tmKV, p);
+    attn_fused_kernel<DH, DROP><<<grid, kAtThreads, smem, s>>>(tmQ, tmKV, p);
     return static_cast<int>(cudaGetLastError());
 }
 
-}  // namespace b200
-
-extern "C" int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh,
-                              float scale, void* stream) {
-    using namespace b200;
+// Argument checks, tensor maps and launch of b200_attention / b200_attention_mc (drop_p in [0, 1); 0 = no dropout).
+static int attention_run(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh, float scale,
+                         float drop_p, unsigned long long drop_seed, void* stream) {
     if (B < 0 || N <= 0 || N > 256 || heads <= 0 || (dh != 64 && dh != 128)) return -1;
     if (B == 0) return 0;
     if (qkv == nullptr || out == nullptr) return -2;
@@ -381,5 +399,27 @@ extern "C" int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld
     p.scale_log2 = scale * 1.4426950408889634f;
     p.out = static_cast<__nv_bfloat16*>(out);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    return dh == 64 ? at_launch<64>(tmQ, tmKV, p, num_sms, s) : at_launch<128>(tmQ, tmKV, p, num_sms, s);
+    if (drop_p > 0.f) {
+        p.drop_thresh = dropout_threshold(drop_p);
+        p.drop_scale = 1.0f / (1.0f - drop_p);
+        p.drop_seed_lo = static_cast<unsigned int>(drop_seed);
+        p.drop_seed_hi = static_cast<unsigned int>(drop_seed >> 32);
+        return dh == 64 ? at_launch<64, true>(tmQ, tmKV, p, num_sms, s) : at_launch<128, true>(tmQ, tmKV, p, num_sms, s);
+    }
+    return dh == 64 ? at_launch<64, false>(tmQ, tmKV, p, num_sms, s) : at_launch<128, false>(tmQ, tmKV, p, num_sms, s);
+}
+
+}  // namespace b200
+
+extern "C" int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh,
+                              float scale, void* stream) {
+    return b200::attention_run(qkv, qkv_ld, out, out_ld, B, N, heads, dh, scale, 0.f, 0, stream);
+}
+
+// b200_attention with nn.Dropout(drop_p) on the softmax probabilities (MC-dropout inference): the row sums stay those
+// of the undropped softmax, kept probabilities are scaled by 1 / (1 - drop_p).  drop_p == 0 runs b200_attention.
+extern "C" int b200_attention_mc(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh,
+                                 float scale, float drop_p, unsigned long long drop_seed, void* stream) {
+    if (!(drop_p >= 0.f && drop_p < 1.f)) return -19;  // NaN fails both comparisons
+    return b200::attention_run(qkv, qkv_ld, out, out_ld, B, N, heads, dh, scale, drop_p, drop_seed, stream);
 }

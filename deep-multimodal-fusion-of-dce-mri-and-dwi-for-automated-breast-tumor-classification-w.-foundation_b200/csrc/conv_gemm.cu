@@ -66,7 +66,8 @@ struct ConvGemmParams {
     int share_box;         // BN = 256: a warp's two 64-column output boxes share one 4 KB staging slot (one more ring stage)
     // MC-dropout (mode 3): element (pixel, channel) of the segments selected by drop_seg (bit 0 = first output,
     // bit 1 = second) is zeroed when Philox4x32-7(seed; pixel * Cout + channel) < drop_thresh, else scaled by
-    // drop_scale = 1 / (1 - p).  Applied after the activation, before the store / channel sums.
+    // drop_scale = 1 / (1 - p).  Applied after the activation, before the store / channel sums.  Mode 4 (the fp32
+    // epilogue of b200_linear_mc) applies the same rule before the residual add.
     unsigned int drop_thresh;
     float drop_scale;
     unsigned int drop_seed_lo, drop_seed_hi;
@@ -149,11 +150,28 @@ struct Tile {
 
 // The epilogue GELU is common.cuh's gelu_fast2 (tanh form on MUFU.TANH, two elements per packed instruction).
 
+// nn.Dropout in MC-dropout inference (reference train_fusion.py:478-481: dropout modules in train mode, BatchNorm
+// frozen) on the 32 columns [n0, n0 + 32) of row `pix`: one Philox call yields the keep decisions of 4 consecutive
+// channels
+__device__ __forceinline__ void dropout_chunk(float (&v)[kChunk], long long pix, int n0, const ConvGemmParams& p) {
+    const unsigned long long e0 = static_cast<unsigned long long>(pix) * p.Cout + n0;
+#pragma unroll
+    for (int j = 0; j < kChunk / 4; ++j) {
+        const uint4 rnd = philox4x32_7(e0 / 4 + j, p.drop_seed_lo, p.drop_seed_hi);
+        v[4 * j + 0] = rnd.x < p.drop_thresh ? 0.f : v[4 * j + 0] * p.drop_scale;
+        v[4 * j + 1] = rnd.y < p.drop_thresh ? 0.f : v[4 * j + 1] * p.drop_scale;
+        v[4 * j + 2] = rnd.z < p.drop_thresh ? 0.f : v[4 * j + 2] * p.drop_scale;
+        v[4 * j + 3] = rnd.w < p.drop_thresh ? 0.f : v[4 * j + 3] * p.drop_scale;
+    }
+}
+
 // Epilogue features are compile-time so that the per-element instruction stream carries no flag tests:
 //   RES  0 none, 1 residual added before the activation, 2 after it
 //   GAP  per-case channel sums          NDOT 0, or 1 / 9 fused per-pixel dot products (no map store)
 //   MODE 0 standard; 1 row softmax numerator: out = exp(alpha*acc - rowmax) as bf16, 1/rowsum to rowsum_inv
-//        (the whole row lives in one N tile; the division is deferred to the consumer GEMM's rowscale)
+//        (the whole row lives in one N tile; the division is deferred to the consumer GEMM's rowscale);
+//        2 fp32 residual / output (b200_linear); 3 MC dropout after the activation; 4 = 2 with MC dropout before the
+//        residual add (b200_linear_mc)
 //   PAIR (BN = 128 only): a CTA works on TWO consecutive M tiles of the same N tile at once - 256 x 128 outputs: per
 //        64-deep k-block the weight slab is loaded once and feeds two MMAs (one per M tile, each with its own TMEM
 //        accumulator), so a stage moves 48 KB for 2 x (128 x 128 x 64) MACs instead of 64 KB.  128 x 128 tiles were
@@ -460,7 +478,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         const int half = ew >> 2;  // column half: columns [half*BN/2, (half+1)*BN/2)
         const int colw0 = half * T::kColsPerWarp;
         const bool share = p.share_box != 0;  // warp-uniform; set by the host for BN = 256 plain-output launches only
-        uint8_t* const obuf0 = s_union + ew * (MODE == 2 ? kF32BlockBytes : (share ? T::kBoxBytes : T::kWarpBoxBytes));
+        uint8_t* const obuf0 = s_union + ew * ((MODE == 2 || MODE == 4) ? kF32BlockBytes : (share ? T::kBoxBytes : T::kWarpBoxBytes));
         const int obuf_flip = p.obuf2 ? 8 * T::kWarpBoxBytes : 0;  // second set of boxes (all 8 warps') behind the first
         int obuf_sel = 0;
         uint8_t* const rbuf = smem + p.off_rbox + ew * T::kWarpBoxBytes;
@@ -472,7 +490,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         const int row_off = lane * T::kRowBytes;
         const bool tma_epi = p.tma_epi != 0;
         // fp32 residual / output (never TMA-staged): transpose through the warp's staging box when it is large enough
-        constexpr bool kF32 = MODE == 2;  // the fp32 code exists only in the instantiations b200_linear uses for it
+        constexpr bool kF32 = MODE == 2 || MODE == 4;  // the fp32 code exists only in the instantiations b200_linear uses
         constexpr bool kTransposeF32 = true;  // the host plans 8 transposition blocks for mode 2
         int acc = 0;
         uint32_t acc_phase = 0;
@@ -705,6 +723,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
                             }
                         }
+                        if (MODE == 4) dropout_chunk(v, pix, n0, p);  // res + drop(act(acc * scale + bias))
                         if (kTransposeF32) {
                             // Coalesced: one warp instruction reads 4 rows x 128 B (8 lanes x 16 B per row), the
                             // 32 x 32 block goes through this warp's (otherwise unused) staging box so that every
@@ -837,19 +856,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
                     }
                 }
-                if (MODE == 3 && (p.drop_seg & (seg2 ? 2 : 1))) {
-                    // nn.Dropout in MC-dropout inference (reference train_fusion.py:478-481: dropout modules in train
-                    // mode, BatchNorm frozen): one Philox call yields the keep decisions of 4 consecutive channels
-                    const unsigned long long e0 = static_cast<unsigned long long>(pix) * p.Cout + n0;
-#pragma unroll
-                    for (int j = 0; j < kChunk / 4; ++j) {
-                        const uint4 rnd = philox4x32_7(e0 / 4 + j, p.drop_seed_lo, p.drop_seed_hi);
-                        v[4 * j + 0] = rnd.x < p.drop_thresh ? 0.f : v[4 * j + 0] * p.drop_scale;
-                        v[4 * j + 1] = rnd.y < p.drop_thresh ? 0.f : v[4 * j + 1] * p.drop_scale;
-                        v[4 * j + 2] = rnd.z < p.drop_thresh ? 0.f : v[4 * j + 2] * p.drop_scale;
-                        v[4 * j + 3] = rnd.w < p.drop_thresh ? 0.f : v[4 * j + 3] * p.drop_scale;
-                    }
-                }
+                if ((MODE == 3 && (p.drop_seg & (seg2 ? 2 : 1))) || (MODE == 4 && RES == 0)) dropout_chunk(v, pix, n0, p);
                 if (DOT) {
 #pragma unroll
                     for (int k = 0; k < NDOT; ++k) {
@@ -1100,6 +1107,11 @@ static int dispatch(int res_mode, bool gap, int ndot, int mode, const CUtensorMa
     }
     if (mode == 2) {  // fp32 residual stream and / or fp32 output (b200_linear)
         if constexpr (!WS) {
+            if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM && p.drop_seg != 0) {  // b200_linear_mc
+                if (res_mode == 0) B200_GO(0, false, 0, 4);
+                if (res_mode == 2) B200_GO(2, false, 0, 4);
+                return -14;
+            }
             if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM) {
                 if (res_mode == 0) B200_GO(0, false, 0, 2);
                 if (res_mode == 1) B200_GO(1, false, 0, 2);
@@ -1580,9 +1592,9 @@ extern "C" int b200_conv_gemm_mc(const void* x, int x_ld, const void* w, const f
                             stream);
 }
 
-extern "C" int b200_linear(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
-                           const void* res, int res_f32, int res_mode, int act, void* out, int out_f32,
-                           void* stream) {
+static int linear_launch(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
+                         const void* res, int res_f32, int res_mode, int act, void* out, int out_f32,
+                         b200::DropoutArgs drop, void* stream) {
     using namespace b200;
     if (x == nullptr || w == nullptr || out == nullptr || M <= 0 || M > 0x7fffffffLL) return -1;
     if (K % 64 != 0 || N % 64 != 0) return -2;
@@ -1621,7 +1633,40 @@ extern "C" int b200_linear(const void* x, long long M, int K, const void* w, int
     j.a = View4{x, {K, M, 1, 1}, {K, 0, 0}};
     j.out = View4{out, {N, M, 1, 1}, {N, 0, 0}};
     j.res = View4{res, {N, M, 1, 1}, {N, 0, 0}};
-    return run_job(p, j, (p.res_f32 || p.out_f32) ? 2 : 0, false, static_cast<cudaStream_t>(stream));
+    int mode = (p.res_f32 || p.out_f32) ? 2 : 0;
+    if (drop.seg != 0) {  // fp32 epilogue: mode 2 with the dropout instantiations (4); bf16 without residual: mode 3
+        if (mode == 0) mode = 3;
+        p.drop_thresh = dropout_threshold(drop.p);
+        p.drop_scale = 1.0f / (1.0f - drop.p);
+        p.drop_seed_lo = static_cast<unsigned int>(drop.seed);
+        p.drop_seed_hi = static_cast<unsigned int>(drop.seed >> 32);
+        p.drop_seg = drop.seg;
+    }
+    return run_job(p, j, mode, false, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int b200_linear(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
+                           const void* res, int res_f32, int res_mode, int act, void* out, int out_f32,
+                           void* stream) {
+    return linear_launch(x, M, K, w, N, scale, bias, res, res_f32, res_mode, act, out, out_f32, b200::DropoutArgs{},
+                         stream);
+}
+
+// b200_linear with MC dropout before the residual add: out = res + drop(act(acc * scale + bias)).
+extern "C" int b200_linear_mc(const void* x, long long M, int K, const void* w, int N, const float* scale,
+                              const float* bias, const void* res, int res_f32, int res_mode, int act, void* out,
+                              int out_f32, float drop_p, unsigned long long drop_seed, void* stream) {
+    if (!b200::dropout_args_valid(drop_p, 1)) return -19;
+    // the residual must be fp32 (a bf16 one goes through mode 3, whose dropout sits after the residual), and added
+    // after the activation: res_mode 1 is accepted without one, where it is the same as 2
+    if (res_mode != 0 && (res_f32 == 0 || (res_mode == 1 && act != 0))) return -19;
+    if (drop_p == 0.f) return b200_linear(x, M, K, w, N, scale, bias, res, res_f32, res_mode, act, out, out_f32, stream);
+    b200::DropoutArgs d;
+    d.p = drop_p;
+    d.seed = drop_seed;
+    d.seg = 1;
+    return linear_launch(x, M, K, w, N, scale, bias, res, res_f32, res_mode == 1 ? 2 : res_mode, act, out, out_f32, d,
+                         stream);
 }
 
 extern "C" int b200_gemm_batched(const b200_gemm_desc* d, void* stream) {

@@ -580,12 +580,24 @@ def _transformer_pack(stage, out_proj, dev):
             "wfc1": blk.mlp.fc1.weight.detach().to(dev, torch.bfloat16).contiguous(), "bfc1": _f32(blk.mlp.fc1.bias, dev),
             "wfc2": blk.mlp.fc2.weight.detach().to(dev, torch.bfloat16).contiguous(), "sfc2": g2,
             "bfc2": (g2 * _f32(blk.mlp.fc2.bias, dev)).contiguous(),
+            # the block's nn.Dropout modules, read at every forward: MC-dropout inference switches them per module
+            "attn_drop": at.attn_drop, "proj_drop": at.proj_drop, "mlp_drop": blk.mlp.drop,
         })
     return tr
 
 
-def _transformer_stage(tr, x):
+def _transformer_dropouts(tr):
+    """True when some nn.Dropout of the packed transformer stage is in train mode with p > 0 (MC dropout)."""
+    return any(m.training and m.p > 0 for ly in tr["layers"] for m in (ly["attn_drop"], ly["proj_drop"], ly["mlp_drop"]))
+
+
+def _transformer_stage(tr, x, drop=None):
     """x [B,H,W,C] bf16 NHWC -> (f3 [B,H/2,W/2,c3] bf16, per-case channel sums of f3).
+
+    `drop(segments, p)` (the encoder's per-launch seed stream, MC-dropout inference) -> (p, seed, segments): every
+    nn.Dropout of a block that is in train mode with p > 0 applies inside the launch it follows, timm's placement
+    (DESIGN.md section 2): attn_drop on the softmax probabilities, proj_drop on proj(o) before LayerScale and the
+    residual, mlp.drop after the GELU and again on fc2's output before LayerScale and the residual.
 
     Pre-norm blocks exactly as transformer_model.py:68-133 (eval: dropout is identity); every matmul runs on
     the tcgen05 GEMM kernel: the patch embedding as a 2x2/stride-2 implicit GEMM, Q.K^T per head with the
@@ -608,18 +620,22 @@ def _transformer_stage(tr, x):
     qkv = torch.empty((M, 3 * E), dtype=torch.bfloat16, device=dev)
     o = torch.empty((M, E), dtype=torch.bfloat16, device=dev)
     u = torch.empty((M, 4 * E), dtype=torch.bfloat16, device=dev)
+
+    def dr(mod):  # (p, seed) of one launch for an active Dropout module, else None
+        return drop(1, float(mod.p))[:2] if drop is not None and mod.training and mod.p > 0 else None
+
     for ly in tr["layers"]:
         heads, dh = ly["heads"], ly["dh"]
         nat.layernorm(t, *ly["ln1"], out=h)
         nat.linear(h, ly["wqkv"], bias=ly["bqkv"], out=qkv)
-        nat.attention(qkv, o, B, N, heads, dh)  # transformer_model.py:101-112 in one launch
+        nat.attention(qkv, o, B, N, heads, dh, dropout=dr(ly["attn_drop"]))  # transformer_model.py:101-112 in one launch
         last = ly is tr["layers"][-1]
         t2 = nat.linear_f32(o, ly["wproj"], scale=ly["sproj"], bias=ly["bproj"], res=t, res_mode=2,
-                            out_dtype=torch.float32)
+                            out_dtype=torch.float32, dropout=dr(ly["proj_drop"]))
         nat.layernorm(t2, *ly["ln2"], out=h)
-        nat.linear(h, ly["wfc1"], bias=ly["bfc1"], act=1, out=u)
+        nat.linear(h, ly["wfc1"], bias=ly["bfc1"], act=1, out=u, dropout=dr(ly["mlp_drop"]))
         t = nat.linear_f32(u, ly["wfc2"], scale=ly["sfc2"], bias=ly["bfc2"], res=t2, res_mode=2,
-                           out_dtype=torch.bfloat16 if last else torch.float32)
+                           out_dtype=torch.bfloat16 if last else torch.float32, dropout=dr(ly["mlp_drop"]))
     c3 = tr["out_w"].shape[0]
     gap = torch.zeros((B, c3), dtype=torch.float32, device=dev)
     f3 = nat.conv_gemm(t.view(B, Ht, Wt, E), tr["out_w"], taps=1, bias=tr["out_b"], gap=gap)
@@ -802,10 +818,13 @@ class ModelMaskHeadBackbone(_PackedWeightsMixin, nn.Module):
 
     def _mc_dropout_p(self):
         """MC-dropout inference as the reference arms it (train_fusion.py:445-481): the module is in eval mode,
-        BatchNorm frozen, but its nn.Dropout sub-modules have been put in train mode.  Returns p (0 = off)."""
-        for mod in self.modules():
-            if isinstance(mod, nn.Dropout) and mod.training and mod.p > 0:
-                return float(mod.p)
+        BatchNorm frozen, but its nn.Dropout sub-modules have been put in train mode.  Returns the p of the CNN
+        blocks' dropouts (0 = off); the hybrid transformer stage's own dropouts (p = 0.1) are read per module."""
+        blocks = [self.block1, self.block2] + ([] if self.use_hybrid_transformer else [self.block3])
+        for blk in blocks:
+            for mod in blk.modules():
+                if isinstance(mod, nn.Dropout) and mod.training and mod.p > 0:
+                    return float(mod.p)
         return 0.0
 
     # ---------------------------------------------------------------- packing ----
@@ -1057,22 +1076,24 @@ class ModelMaskHeadBackbone(_PackedWeightsMixin, nn.Module):
 
             return encoder_train_forward_autograd(self, x)
         p_drop = self._mc_dropout_p()
-        if p_drop > 0 and self.use_hybrid_transformer:
-            raise NotImplementedError("MC dropout with the hybrid transformer stage (its attention / MLP dropouts)")
+        dev = x.device
+        pk = self._packed(dev)
         self._drop = None
-        if p_drop > 0:  # per-launch seeds: (model seed, forward count, launch count)
+        if p_drop > 0 or (self.use_hybrid_transformer and _transformer_dropouts(pk["tr"])):
+            # per-launch seeds: (model seed, forward count, launch count)
             self._mc_calls += 1
             base = (self._mc_seed * 0x9E3779B97F4A7C15 + self._mc_calls * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF
             counter = [0]
 
-            def _drop(segments=1):
+            def _drop(segments=1, p=p_drop):
+                """(p, seed, segments) of the next dropout launch, or None when p is 0 (p defaults to the CNN blocks')."""
+                if p <= 0:
+                    return None
                 counter[0] += 1
-                return (p_drop, (base + counter[0] * 0x94D049BB133111EB) & 0xFFFFFFFFFFFFFFFF, segments)
+                return (p, (base + counter[0] * 0x94D049BB133111EB) & 0xFFFFFFFFFFFFFFFF, segments)
 
             self._drop = _drop
         full = self.aux_mode == "full"
-        dev = x.device
-        pk = self._packed(dev)
         x = x.contiguous().float()
         B, C, H, W = x.shape
         mod_attn = None
@@ -1100,7 +1121,7 @@ class ModelMaskHeadBackbone(_PackedWeightsMixin, nn.Module):
             if input_norm is not None and plane_mean is None:
                 raise ValueError("input_norm needs the plane means of the normalised values (fused_params returns both)")
             nat.stem(x, stride, plane_mean, se, st["w"], st["s"], st["b"], st["n_skip"], st["n_mid"], skip1, mid1,
-                     mod_attn, dropout=self._drop(1)[:2] if self._drop else None, input_norm=input_norm)
+                     mod_attn, dropout=self._drop(1)[:2] if self._drop and p_drop > 0 else None, input_norm=input_norm)
             f1, r1, _, _ = self._run_block(pk["b1"], mid1, skip1, full)
 
         mask_pred = attn_map = None
@@ -1113,7 +1134,7 @@ class ModelMaskHeadBackbone(_PackedWeightsMixin, nn.Module):
         if self.mask_enabled and self.mask_stage == "f2":                       # reference :681-685
             mask_pred, attn_map = self._mask_stage(pk["mask"], f2, f1)
         if self.use_hybrid_transformer:
-            f3, gap3 = _transformer_stage(pk["tr"], f2)  # reference :702-703
+            f3, gap3 = _transformer_stage(pk["tr"], f2, self._drop)  # reference :702-703
             gate3 = None
         else:
             f3_in = f2

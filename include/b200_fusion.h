@@ -109,6 +109,17 @@ int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, in
                    void* stream);
 
 /*
+ * b200_attention with the attention dropout of MC-dropout inference (nn.Dropout(drop_p) in train mode on the softmax
+ * probabilities, code/transformer_model.py:109-116): probability (b, h, n, j) is kept when word j % 4 of
+ * Philox4x32-7(drop_seed; ((b * heads + h) * N + n) * 64 + j / 4) >= drop_p * 2^32, else it is 0; the row sums are
+ * those of the undropped softmax and the kept probabilities are scaled by 1 / (1 - drop_p).  The decision depends
+ * only on the seed and the indices.  drop_p == 0 runs b200_attention.  Returns -19 unless 0 <= drop_p < 1 (nothing
+ * launched), else as b200_attention.
+ */
+int b200_attention_mc(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh, float scale,
+                      float drop_p, unsigned long long drop_seed, void* stream);
+
+/*
  * Batched GEMM on the same tcgen05 kernel: for every (batch, head)
  *     out[m, n] = epilogue( sum_k A[m, k] * B[n, k] ),   A, B bf16 K-major, fp32 accumulation.
  * This is how the transformer blocks run (code/transformer_model.py:98-116): Q.K^T per head
@@ -172,6 +183,19 @@ int b200_vit_feature(const float* t, int B, int n_patch, int E, void* out, int o
  */
 int b200_linear(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
                 const void* res, int res_f32, int res_mode, int act, void* out, int out_f32, void* stream);
+
+/*
+ * b200_linear with nn.Dropout(drop_p) in train mode (MC-dropout inference) before the residual add:
+ *     out = res + drop(act(acc * scale + bias))
+ * Element (row, col) is dropped when Philox4x32-7(drop_seed; row * N + col) < drop_p * 2^32 (one call decides four
+ * consecutive columns; the rule of b200_conv_gemm_mc), the kept ones are scaled by 1 / (1 - drop_p).  Supported:
+ * an fp32 residual (res_mode 1 with act 0, or res_mode 2) with fp32 or bf16 output, and no residual.  Returns -19
+ * unless 0 <= drop_p < 1, and for a bf16 residual or res_mode 1 with an activation (nothing launched); drop_p == 0
+ * runs b200_linear.  Other returns as b200_linear.
+ */
+int b200_linear_mc(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
+                   const void* res, int res_f32, int res_mode, int act, void* out, int out_f32, float drop_p,
+                   unsigned long long drop_seed, void* stream);
 
 /* out[b,h,w] = bias + sum_k d[(b,h+ky-1,w+kx-1)][k], zero padded: finishes a 3x3 C->1 conv from tap dots. */
 int b200_tapsum(const float* d, int B, int H, int W, const float* bias, float* out, void* stream);
