@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # csrc/build.sh links the library at <repo>/lib/libb200fusion.so: a short path without the dots and dashes of the
 # package directory name, which is the path string dlopen sees.
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb200fusion.so")
-ABI_VERSION = 22
+ABI_VERSION = 23
 
 _lib = None
 
@@ -92,7 +92,6 @@ _P, _I, _F, _LL = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 # name -> argtypes; must list every symbol include/b200_fusion.h declares (tests check this).
 SIGNATURES = {
     "b200_abi_version": [],
-    "b200_conv_gemm": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _P, _I, _I, _I, _I, _I, _I, _P],
     "b200_conv_gemm_ex": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _P, _I, _P, _I, _I, _P, _I, _F, _P, _I, _I, _I,
                           _I, _I, _I, _I, _I, _P],
     "b200_conv_gemm_mc": [_P, _I, _P, _P, _P, _P, _I, _I, _I, _P, _I, _I, _P, _I, _P, _I, _I, _P, _I, _F, _P, _I, _I, _I,
@@ -116,11 +115,9 @@ SIGNATURES = {
     "b200_stem_ex": [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _F, _F, _P, _I, _P],
     "b200_stem_mc": [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P, _F, _F, _P, _I, _F,
                      C.c_ulonglong, _P],
-    "b200_nyul_transform": [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P],
     "b200_nyul_transform_ex": [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P],
     "b200_plane_mean": [_P, _I, _I, _P, _P],
     "b200_case_max_scale": [_P, _I, _LL, _P, _P],
-    "b200_stem": [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P],
     "b200_se_gate": [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P],
     "b200_scale_map": [_P, _P, _I, _I, _I, _P, _P, _P, _P],
     "b200_conv3x3_c1": [_P, _I, _I, _I, _I, _P, _P, _P, _P],
@@ -132,7 +129,6 @@ SIGNATURES = {
     "b200_adaptive_pool": [_P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "b200_add_maps": [_P, _P, _LL, _P, _P],
     "b200_adc_map": [_P, _I, _I, _I, _P, _F, _P, _P],
-    "b200_conv7x7_s2": [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P],
     "b200_maxpool3x3_s2": [_P, _I, _I, _I, _I, _P, _P],
     "b200_im2col7x7_s2": [_P, _P, _I, _I, _I, _I, _I, _P, _P],
     "b200_flip_planes": [_P, _P, _LL, _I, _I, _I, _I, _P],
@@ -490,15 +486,6 @@ def adc_map(x, bvals, eps=1e-6):
     out = torch.empty((B, 1, H, W), dtype=torch.float32, device=x.device)
     _call("b200_adc_map", None, _ptr(x), B, C_, H * W, _ptr(bvals), float(eps), _ptr(out), _stream())
     return out
-
-
-def conv7x7_s2(x, gate, wt, scale, bias):
-    """ResNet stem: x [B,C,H,W] fp32 -> relu(bn(conv7x7/s2)) as bf16 NHWC [B,H/2,W/2,64]; wt [C,49,64] fp32."""
-    x = x.contiguous().float()
-    B, C_, H, W = x.shape
-    y = torch.empty((B, H // 2, W // 2, 64), dtype=torch.bfloat16, device=x.device)
-    _call("b200_conv7x7_s2", None, _ptr(x), _ptr(gate), B, C_, H, W, _ptr(wt), _ptr(scale), _ptr(bias), _ptr(y), _stream())
-    return y
 
 
 def im2col7x7_s2(x, gate, kp):

@@ -12,9 +12,9 @@ __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf
 
 // GELU of every stored inference activation: 0.5 x (1 + tanh(x (c0 + c1 x^2))) with the hardware tanh (MUFU.TANH),
 // two elements per instruction on the packed fp32x2 pipe: 5 packed instructions + 2 MUFU per pair.  The 8-term
-// polynomial erf it replaces (kept below as gelu_erf_poly2; exact to 9e-5) cost 13 packed + 4 FMNMX per pair, and the
-// GEMM epilogues of the 1x1 layers are instruction-issue bound: block tail 0.709 -> 0.634 ms, C3 step -5 %, C4 -3 %
-// on the same box (tools/ab_gelu.sh).  Deviation from nn.GELU() (erf): <= 4.7e-4 from the tanh form plus the 2^-11
+// polynomial erf it replaced (exact to 9e-5) cost 13 packed + 4 FMNMX per pair, and the GEMM epilogues of the 1x1
+// layers are instruction-issue bound: block tail 0.709 -> 0.634 ms, C3 step -5 %, C4 -3 % on the same box.
+// Deviation from nn.GELU() (erf): <= 4.7e-4 from the tanh form plus the 2^-11
 // relative error of MUFU.TANH on (1 + tanh), together <= 1.2e-3 ABSOLUTE (largest around x = -3 .. -2, where
 // gelu ~ -0.01 .. -0.05) - below the bf16 rounding step of every output with |y| >= 0.3, and 2e-4 of a typical map's
 // range.  Measured effect on parity with the trained weights: fusion logits 5.6e-3 (was 5.7e-3), argmax agreement
@@ -29,28 +29,6 @@ __device__ __forceinline__ float2 gelu_fast2(float2 x) {
     const float2 h = __fmul2_rn(x, make_float2(0.5f, 0.5f));
     return __ffma2_rn(h, th, h);
 }
-
-// The erf form: erf(z) ~= z * P(z^2) on |z| <= 3 (8-term odd minimax polynomial, |erf error| < 9e-5, continuous with
-// +-1 at the clamp).  Not on the product path any more; -DB200_GELU_ERF builds the library with it for A/B runs.
-__device__ __forceinline__ float2 gelu_erf_poly2(float2 x) {
-    float2 z = __fmul2_rn(x, make_float2(0.70710678118654752f, 0.70710678118654752f));
-    z.x = fminf(fmaxf(z.x, -3.0f), 3.0f);
-    z.y = fminf(fmaxf(z.y, -3.0f), 3.0f);
-    const float2 t = __fmul2_rn(z, z);
-    float2 p = make_float2(-3.901667185e-07f, -3.901667185e-07f);
-    p = __ffma2_rn(p, t, make_float2(1.668003461e-05f, 1.668003461e-05f));
-    p = __ffma2_rn(p, t, make_float2(-3.086500801e-04f, -3.086500801e-04f));
-    p = __ffma2_rn(p, t, make_float2(3.281538375e-03f, 3.281538375e-03f));
-    p = __ffma2_rn(p, t, make_float2(-2.256273106e-02f, -2.256273106e-02f));
-    p = __ffma2_rn(p, t, make_float2(1.075116023e-01f, 1.075116023e-01f));
-    p = __ffma2_rn(p, t, make_float2(-3.730817735e-01f, -3.730817735e-01f));
-    p = __ffma2_rn(p, t, make_float2(1.127865076e+00f, 1.127865076e+00f));
-    const float2 h = __fmul2_rn(x, make_float2(0.5f, 0.5f));
-    return __ffma2_rn(h, __fmul2_rn(z, p), h);
-}
-#ifdef B200_GELU_ERF
-#define gelu_fast2 gelu_erf_poly2
-#endif
 
 template <typename T>
 __device__ __forceinline__ T warp_sum(T v) {

@@ -96,7 +96,7 @@ struct ConvGemmParams {
     int obuf2;             // output staging double-buffered per epilogue warp (tile i+1 is staged while the TMA store of
                            // tile i still reads its boxes); 0: one set of boxes, the store is waited for at the next tile
     int pair;              // BN = 128: two M tiles per CTA iteration share one weight slab (conv_gemm_kernel<..., PAIR>)
-    int off_ring, off_bar, off_union, off_rbox, off_sm;  // shared-memory plan (bytes from the 1 KB-aligned base)
+    int off_bar, off_union, off_rbox, off_sm;  // shared-memory plan (bytes from the 1 KB-aligned base)
     int off_aff;           // >= 0: [scale Cout | bias Cout] parked in shared memory once per CTA (BN <= 128 launches);
                            // -1: they are read from global memory per chunk
 };
@@ -128,11 +128,7 @@ constexpr int kMaxStages = 12;
 constexpr int kBarBytes = 512;
 
 // Shared-memory plan, computed on the host (plan_smem) and passed in ConvGemmParams:
-//   [ resident weights (weight-stationary mode) | operand ring | barriers | union{output boxes, tap-dot
-//     buffers} | residual boxes ]
-// Weight-stationary mode (1x1 layers whose whole [BN, K] weight slab fits): the CTA owns one N tile, loads
-// its weights once and only streams activations, so the ring holds 16 KB stages and runs several tiles
-// ahead (the activations of a 1x1 layer come from DRAM, and a 3-stage ring cannot cover that latency).
+//   [ operand ring | barriers | union{output boxes, tap-dot buffers} | residual boxes ]
 template <int BN>
 struct Tile {
     static constexpr int kBBytes = BN * kBlockK * 2;
@@ -177,7 +173,7 @@ __device__ __forceinline__ void dropout_chunk(float (&v)[kChunk], long long pix,
 //        accumulator), so a stage moves 48 KB for 2 x (128 x 128 x 64) MACs instead of 64 KB.  128 x 128 tiles were
 //        shared-memory-feed bound (0.64 PFLOP/s on 3x3 128->128 against 1.24 for the 128 x 256 tiles); four accumulator
 //        stages (512 TMEM columns) keep the epilogue of one pair overlapped with the MMAs of the next.
-template <int BN, bool WS, int RES, bool GAP, int NDOT, int MODE, bool PAIR = false>
+template <int BN, int RES, bool GAP, int NDOT, int MODE, bool PAIR = false>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
@@ -188,10 +184,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // 1 KB alignment by OFFSET (not by rounding the generic address): the compiler keeps the shared state space
     // and emits STS / LDS for the staging traffic instead of generic ST / LD
     uint8_t* smem = smem_raw + ((1024u - (static_cast<uint32_t>(__cvta_generic_to_shared(smem_raw)) & 1023u)) & 1023u);
-    uint8_t* sW = smem;  // resident weights [k_blocks][BN x 64] (WS only)
-    uint8_t* sRing = smem + p.off_ring;
-    static_assert(!PAIR || ((BN == 128 || BN == 64) && !WS && MODE == 0), "PAIR: BN = 128 / 64, streamed weights, standard epilogue");
-    constexpr int kStageBytes = WS ? kABytes : (PAIR ? 2 * kABytes : kABytes) + T::kBBytes;
+    uint8_t* sRing = smem;
+    static_assert(!PAIR || ((BN == 128 || BN == 64) && MODE == 0), "PAIR: BN = 128 / 64, standard epilogue");
+    constexpr int kStageBytes = (PAIR ? 2 * kABytes : kABytes) + T::kBBytes;
     constexpr int kAcc = PAIR ? 4 : 2;             // accumulator stages in TMEM
     constexpr int kTmemCols = PAIR ? T::kTmemColsPair : T::kTmemCols;
     uint64_t* full = reinterpret_cast<uint64_t*>(smem + p.off_bar);
@@ -199,8 +194,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     uint64_t* tfull = empty + kMaxStages;
     uint64_t* tempty = tfull + 4;
     uint64_t* resbar = tempty + 4;  // [kNumEpiWarps][2] residual-box arrival, one per epilogue warp and box
-    uint64_t* wbar = resbar + 2 * kNumEpiWarps;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(wbar + 1);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(resbar + 2 * kNumEpiWarps);
     uint8_t* s_union = smem + p.off_union;
     float* s_dotw = reinterpret_cast<float*>(s_union);  // [NDOT][BN]       (dot mode)
     float* s_dots = s_dotw + NDOT * BN;                 // [2][128][NDOT]   (dot mode)
@@ -208,20 +202,13 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
     const int stages = p.stages;
-    // tile walk: WS CTAs keep one N tile and stride over M tiles; otherwise tiles are dealt round-robin, N fastest
-    const int my_n = WS ? static_cast<int>(blockIdx.x) % p.n_tiles : 0;
-    const int m_first = WS ? static_cast<int>(blockIdx.x) / p.n_tiles : 0;
-    const int m_step = WS ? static_cast<int>(gridDim.x) / p.n_tiles : 0;
+    // tile walk: tiles are dealt round-robin, N fastest
     const int total_tiles = PAIR ? ((p.m_tiles + 1) / 2) * p.n_tiles : p.m_tiles * p.n_tiles;  // PAIR: super-tiles
-    const int n_iters = WS ? (p.m_tiles > m_first ? (p.m_tiles - m_first + m_step - 1) / m_step : 0)
-                           : (total_tiles > static_cast<int>(blockIdx.x)
-                                  ? (total_tiles - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) /
-                                        static_cast<int>(gridDim.x)
-                                  : 0);
+    const int n_iters = total_tiles > static_cast<int>(blockIdx.x)
+                            ? (total_tiles - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) /
+                                  static_cast<int>(gridDim.x)
+                            : 0;
 
-    // Programmatic dependent launch: the next kernel of the stream may take this SM the moment this CTA retires (its
-    // own prologue - descriptor prefetch, barrier init, TMEM allocation - then overlaps the tail of this grid) ...
-    griddep_launch_dependents();
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmA);
         tma_prefetch_desc(&tmB);
@@ -241,13 +228,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             mbar_init(&tempty[s], MODE == 1 ? kNumEpiWarps / 2 : kNumEpiWarps);  // mode 1: one warp set per stage
         }
         for (int s = 0; s < 2 * kNumEpiWarps; ++s) mbar_init(&resbar[s], 1);
-        mbar_init(wbar, 1);
         fence_mbar_init();
     }
     if (warp == 2) tmem_alloc<kTmemCols>(tmem_slot);
-    // ... and nothing below (the first global read is the tap-dot weight staging) runs before the previous grids of the
-    // stream have completed and flushed
-    griddep_wait();
     if (DOT && warp >= kEpiWarp0) {
         for (int i = threadIdx.x - kEpiWarp0 * 32; i < NDOT * BN; i += kNumEpiWarps * 32) s_dotw[i] = p.dot_w[i];
     }
@@ -258,18 +241,13 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
     if (warp == 0) {
         if (lane == 0 && n_iters > 0) {
-            if (WS) {  // the CTA's whole weight slab, once
-                mbar_arrive_expect_tx(wbar, p.k_blocks * T::kBBytes);
-                for (int kb = 0; kb < p.k_blocks; ++kb)
-                    tma_load_2d(sW + kb * T::kBBytes, &tmB, wbar, kb * kBlockK, my_n * BN);
-            }
             int stage = 0;
             uint32_t phase = 0;
-            int tile = blockIdx.x, m_tile = m_first;
-            for (int it = 0; it < n_iters; ++it, tile += gridDim.x, m_tile += m_step) {
+            int tile = blockIdx.x;
+            for (int it = 0; it < n_iters; ++it, tile += gridDim.x) {
                 const int tq = fd_div(p.fd_ntiles, tile);
-                const int n_tile = WS ? my_n : tile - tq * p.n_tiles;
-                const int mt = WS ? m_tile : (PAIR ? 2 * tq : tq);
+                const int n_tile = tile - tq * p.n_tiles;
+                const int mt = PAIR ? 2 * tq : tq;
                 int tw0, th0, tb0, tw1 = 0, th1 = 0, tb1 = 0;
                 tile_whb(p, mt, tw0, th0, tb0);
                 const int w0 = tw0 * p.BW, h0 = th0 * p.BH, b = tb0 * p.BB;
@@ -289,16 +267,14 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                         dx = tap & 1;
                     }
                     mbar_wait(&empty[stage], phase ^ 1);
-                    mbar_arrive_expect_tx(&full[stage], p.a_box_bytes * (has2 ? 2 : 1) + (WS ? 0 : T::kBBytes));
+                    mbar_arrive_expect_tx(&full[stage], p.a_box_bytes * (has2 ? 2 : 1) + T::kBBytes);
                     uint8_t* dst = sRing + stage * kStageBytes;
                     if (p.a_batched) tma_load_4d(dst, &tmA, &full[stage], c0, p.cstride * w0 + dx, p.cstride * h0 + dy, b);
                     else tma_load_4d(dst, &tmA, &full[stage], c0, w0, 0, 0);
                     if (has2) tma_load_4d(dst + kABytes, &tmA, &full[stage], c0, p.cstride * w1 + dx, p.cstride * h1 + dy, b1);
                     constexpr int kBOff = PAIR ? 2 * kABytes : kABytes;
-                    if (!WS) {
-                        if (p.b_mode == 0) tma_load_2d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN);
-                        else tma_load_4d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN, h0, b);
-                    }
+                    if (p.b_mode == 0) tma_load_2d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN);
+                    else tma_load_4d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN, h0, b);
                     if (++stage == stages) {
                         stage = 0;
                         phase ^= 1;
@@ -313,7 +289,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             uint32_t phase = 0;
             int acc = 0;
             uint32_t acc_phase = 0;
-            if (WS) mbar_wait(wbar, 0);
             int tile = blockIdx.x;
             for (int it = 0; it < n_iters; ++it, tile += gridDim.x) {
                 const bool has2 = PAIR && 2 * fd_div(p.fd_ntiles, tile) + 1 < p.m_tiles;
@@ -326,7 +301,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     tc_fence_after();
                     const uint8_t* a_src = sRing + stage * kStageBytes;
                     const uint64_t da = umma_desc_sw128(smem_u32(a_src));
-                    const uint64_t db = umma_desc_sw128(smem_u32(WS ? sW + kb * T::kBBytes : a_src + (PAIR ? 2 * kABytes : kABytes)));
+                    const uint64_t db = umma_desc_sw128(smem_u32(a_src + (PAIR ? 2 * kABytes : kABytes)));
 #pragma unroll
                     for (int k = 0; k < kBlockK / 16; ++k) {
                         // 16 bf16 = 32 bytes along K inside the 128-byte swizzle row -> +2 in 16-byte units
@@ -494,7 +469,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         constexpr bool kTransposeF32 = true;  // the host plans 8 transposition blocks for mode 2
         int acc = 0;
         uint32_t acc_phase = 0;
-        int tile = blockIdx.x, m_walk = m_first;
+        int tile = blockIdx.x;
         // tile-invariant pieces of the row -> pixel map (the TMA box is {64 ch, BW, BH, BB}, rows in that order)
         const int trow = q * 32 + lane;
         const int r_w = trow % p.BW, r_h = (trow / p.BW) % p.BH, r_b = trow / (p.BW * p.BH);
@@ -523,22 +498,22 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             tma_load_4d(rbuf + bx * T::kBoxBytes, &tmRes, &rbar[bx], nt * BN + colw0 + bx * T::kBoxCols, fw, fh, fb);
         };
         // the CTA's tile sequence: (tile index, sub) -> (N tile, M tile); PAIR walks super-tiles of two M tiles
-        auto tile_nm = [&](int t_idx, int m_idx, int sub, int& nt, int& mt) {
+        auto tile_nm = [&](int t_idx, int sub, int& nt, int& mt) {
             const int tq = fd_div(p.fd_ntiles, t_idx);
-            nt = WS ? my_n : t_idx - tq * p.n_tiles;
-            mt = WS ? m_idx : (PAIR ? 2 * tq + sub : tq);
+            nt = t_idx - tq * p.n_tiles;
+            mt = PAIR ? 2 * tq + sub : tq;
             return mt < p.m_tiles;
         };
         if (RES != 0 && tma_epi && lane == 0 && n_iters > 0) {
             int nt0, mt0;
-            tile_nm(tile, m_walk, 0, nt0, mt0);
+            tile_nm(tile, 0, nt0, mt0);
 #pragma unroll
             for (int bx = 0; bx < T::kBoxesPerWarp; ++bx) res_fetch(nt0, mt0, bx);
         }
-        for (int it = 0; it < n_iters; ++it, tile += gridDim.x, m_walk += m_step) {
+        for (int it = 0; it < n_iters; ++it, tile += gridDim.x) {
           for (int sub = 0; sub < (PAIR ? 2 : 1); ++sub) {
             int n_tile, m_tile;
-            if (!tile_nm(tile, m_walk, sub, n_tile, m_tile)) {  // (PAIR) the absent second tile of an odd count
+            if (!tile_nm(tile, sub, n_tile, m_tile)) {  // (PAIR) the absent second tile of an odd count
                 if (++acc == kAcc) {
                     acc = 0;
                     acc_phase ^= 1;
@@ -548,8 +523,8 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             // the tile this warp handles next (its residual boxes are prefetched while this one is in flight)
             int n_next = 0, m_next = 0;
             bool have_next = false;
-            if (PAIR && sub == 0) have_next = tile_nm(tile, m_walk, 1, n_next, m_next);
-            if (!have_next && it + 1 < n_iters) have_next = tile_nm(tile + gridDim.x, m_walk + m_step, 0, n_next, m_next);
+            if (PAIR && sub == 0) have_next = tile_nm(tile, 1, n_next, m_next);
+            if (!have_next && it + 1 < n_iters) have_next = tile_nm(tile + gridDim.x, 0, n_next, m_next);
             // tile -> (w0, h0, b); this warp's slab = 32 consecutive rows of the tile = a {bw, bh} box in (w, h)
             int tw0, th0, tb0;
             tile_whb(p, m_tile, tw0, th0, tb0);
@@ -1051,93 +1026,71 @@ static EncodeTiledFn get_encode_fn() {
 static int g_num_sms = 0;
 constexpr int kSmemLimit = 227 * 1024;
 
-template <int BN, bool WS, int RES, bool GAP, int NDOT, int MODE, bool PAIR = false>
+template <int BN, int RES, bool GAP, int NDOT, int MODE, bool PAIR = false>
 static int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmOut, const CUtensorMap& tmOut2,
                   const CUtensorMap& tmRes, const ConvGemmParams& p, int smem_bytes, int grid, cudaStream_t stream) {
     static int configured = 0;
     if (smem_bytes > configured) {
-        cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<BN, WS, RES, GAP, NDOT, MODE, PAIR>,
+        cudaError_t e = cudaFuncSetAttribute(conv_gemm_kernel<BN, RES, GAP, NDOT, MODE, PAIR>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
         if (e != cudaSuccess) return static_cast<int>(e);
         configured = smem_bytes;
     }
-    // programmatic stream serialisation: this grid's CTAs may be scheduled while the previous kernel drains; the kernel
-    // itself waits (griddepcontrol.wait, after its prologue) before it touches global memory
-    // Opt-in (B200_PDL=1): measured on the C3 step it is a wash (62.9 k vs 63.4 k cases/s on a power-capped box) - a
-    // conv CTA holds ~200 KB of shared memory, so the next grid's CTA can only move in once this one has retired and
-    // what overlaps is the ~1-2 us launch gap, which the front end already pipelines.
-    static const bool no_pdl = std::getenv("B200_PDL") == nullptr;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(static_cast<unsigned>(grid));
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, conv_gemm_kernel<BN, WS, RES, GAP, NDOT, MODE, PAIR>, tmA, tmB, tmOut,
-                                             tmOut2, tmRes, p);
-    return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
+    conv_gemm_kernel<BN, RES, GAP, NDOT, MODE, PAIR>
+        <<<grid, kThreads, static_cast<size_t>(smem_bytes), stream>>>(tmA, tmB, tmOut, tmOut2, tmRes, p);
+    return static_cast<int>(cudaGetLastError());
 }
 
-template <int BN, bool WS>
+template <int BN>
 static int dispatch(int res_mode, bool gap, int ndot, int mode, const CUtensorMap& tmA, const CUtensorMap& tmB,
                     const CUtensorMap& tmOut, const CUtensorMap& tmOut2, const CUtensorMap& tmRes,
                     const ConvGemmParams& p, int smem_bytes, int grid, cudaStream_t s) {
 #define B200_GO(RES, GAP, DOT, MODE) \
-    return launch<BN, WS, RES, GAP, DOT, MODE>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s)
+    return launch<BN, RES, GAP, DOT, MODE>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s)
     if (mode == 1) {
-        if constexpr (!WS && BN == 256) {
+        if constexpr (BN == 256) {
             if (res_mode == 0 && !gap && ndot == 0) B200_GO(0, false, 0, 1);
         }
         return -14;
     }
     if (mode == 3) {  // MC-dropout epilogue (plain / residual, with or without channel sums)
-        if constexpr (!WS) {
-            if (ndot == 0) {
-                if (res_mode == 0 && gap) B200_GO(0, true, 0, 3);
-                if (res_mode == 0) B200_GO(0, false, 0, 3);
-                if (res_mode == 1 && gap) B200_GO(1, true, 0, 3);
-                if (res_mode == 1) B200_GO(1, false, 0, 3);
-            }
+        if (ndot == 0) {
+            if (res_mode == 0 && gap) B200_GO(0, true, 0, 3);
+            if (res_mode == 0) B200_GO(0, false, 0, 3);
+            if (res_mode == 1 && gap) B200_GO(1, true, 0, 3);
+            if (res_mode == 1) B200_GO(1, false, 0, 3);
         }
         return -14;
     }
     if (mode == 2) {  // fp32 residual stream and / or fp32 output (b200_linear)
-        if constexpr (!WS) {
-            if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM && p.drop_seg != 0) {  // b200_linear_mc
-                if (res_mode == 0) B200_GO(0, false, 0, 4);
-                if (res_mode == 2) B200_GO(2, false, 0, 4);
-                return -14;
-            }
-            if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM) {
-                if (res_mode == 0) B200_GO(0, false, 0, 2);
-                if (res_mode == 1) B200_GO(1, false, 0, 2);
-                if (res_mode == 2) B200_GO(2, false, 0, 2);
-            }
+        if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM && p.drop_seg != 0) {  // b200_linear_mc
+            if (res_mode == 0) B200_GO(0, false, 0, 4);
+            if (res_mode == 2) B200_GO(2, false, 0, 4);
+            return -14;
+        }
+        if (!gap && ndot == 0 && p.H == 1 && p.BW == kBlockM) {
+            if (res_mode == 0) B200_GO(0, false, 0, 2);
+            if (res_mode == 1) B200_GO(1, false, 0, 2);
+            if (res_mode == 2) B200_GO(2, false, 0, 2);
         }
         return -14;
     }
     if (ndot != 0) {
-        if constexpr (BN == 128 && !WS) {
+        if constexpr (BN == 128) {
             // paired M tiles for the N = 128 tap-dot layers too (3x3 128->128 + GELU + nine dots, the reconstruction
             // heads): the unpaired 128 x 128 tiles were shared-memory-feed bound like the plain ones
             if (p.pair && res_mode == 0 && !gap && ndot == 9)
-                return launch<BN, WS, 0, false, 9, 0, true>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s);
+                return launch<BN, 0, false, 9, 0, true>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s);
             if (p.pair) return -14;
         }
-        if constexpr (!WS) {
-            if (res_mode == 0 && !gap && ndot == 9) B200_GO(0, false, 9, 0);
-            if (res_mode == 0 && !gap && ndot == 1) B200_GO(0, false, 1, 0);
-        }
+        if (res_mode == 0 && !gap && ndot == 9) B200_GO(0, false, 9, 0);
+        if (res_mode == 0 && !gap && ndot == 1) B200_GO(0, false, 1, 0);
         return -14;
     }
-    if constexpr ((BN == 128 || BN == 64) && !WS) {
+    if constexpr (BN == 128 || BN == 64) {
         if (p.pair) {
 #define B200_GO_PAIR(RES, GAP) \
-    return launch<BN, WS, RES, GAP, 0, 0, true>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s)
+    return launch<BN, RES, GAP, 0, 0, true>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s)
             if (res_mode == 0 && gap) B200_GO_PAIR(0, true);
             if (res_mode == 0) B200_GO_PAIR(0, false);
             if (res_mode == 1 && gap) B200_GO_PAIR(1, true);
@@ -1181,25 +1134,23 @@ static const float* identity_affine(bool ones) {
 
 static inline int align1k(int v) { return (v + 1023) & ~1023; }
 
-// Lays out shared memory for (BN, weight-stationary?) and returns the total dynamic size, or -1 if the
-// configuration does not fit / leaves fewer than 3 ring stages.
-static int plan_smem(ConvGemmParams& p, int BN, bool ws, bool has_out, bool has_res, int ndot, int mode,
-                     bool share_box = false, bool pair = false) {
+// Lays out shared memory for BN and returns the total dynamic size, or -1 if the configuration does not fit / leaves
+// fewer than 3 ring stages.
+static int plan_smem(ConvGemmParams& p, int BN, bool has_out, bool has_res, int ndot, int mode, bool share_box,
+                     bool pair) {
     const int b_bytes = BN * kBlockK * 2;
-    const int stage_bytes = ws ? kABytes : (pair ? 2 * kABytes : kABytes) + b_bytes;
+    const int stage_bytes = (pair ? 2 * kABytes : kABytes) + b_bytes;
     const int box_all = kBlockM * BN * 2;  // 8 warps x (32 rows x BN/2 columns) of bf16
     const int dot_bytes = ndot * BN * 4 + 2 * kBlockM * ndot * 4;
     // mode 2 (fp32 epilogue) needs only the eight 32 x 33-word transposition blocks
     // One-k-block-deep layers (1x1, Cin <= 256) are epilogue bound, and with one set of staging boxes every tile's
     // epilogue starts by waiting for the previous tile's TMA store to finish reading them: a second set hides that.
-    static const bool no_obuf2 = std::getenv("B200_NO_OBUF2") != nullptr;  // A/B measurements
-    const bool want2 = !no_obuf2 && !ws && BN <= 128 && (mode == 0 || mode == 3) && has_out && !share_box && ndot == 0 &&
-                       p.tma_epi && p.k_blocks <= 4;
+    const bool want2 = BN <= 128 && (mode == 0 || mode == 3) && has_out && !share_box && ndot == 0 && p.tma_epi &&
+                       p.k_blocks <= 4;
     int out_stage = mode == 2 ? 8 * kF32BlockBytes : (share_box ? box_all / 2 : box_all);
     p.obuf2 = 0;
     if (want2) {
-        const int fixed2 = (ws ? align1k(p.k_blocks * b_bytes) : 0) + align1k(kBarBytes) + align1k(2 * box_all) +
-                           (has_res ? align1k(box_all) : 0) + 1024;
+        const int fixed2 = align1k(kBarBytes) + align1k(2 * box_all) + (has_res ? align1k(box_all) : 0) + 1024;
         if ((kSmemLimit - fixed2) / stage_bytes >= 4) {
             out_stage = 2 * box_all;
             p.obuf2 = 1;
@@ -1208,18 +1159,13 @@ static int plan_smem(ConvGemmParams& p, int BN, bool ws, bool has_out, bool has_
     const int union_bytes = align1k(ndot ? dot_bytes : (has_out ? out_stage : 0));
     const int rbox_bytes = has_res ? align1k(box_all) : 0;
     const int sm_bytes = mode == 1 ? align1k(8 * kBlockM * 4) : 0;  // row max / row sum exchange
-    const int resident = ws ? align1k(p.k_blocks * b_bytes) : 0;
-    static const bool no_aff = std::getenv("B200_NO_AFF_SMEM") != nullptr;  // A/B measurements
-    const int aff_bytes = ((BN <= 128 || p.k_blocks <= 4) && p.Cout <= 2048 && mode != 1 && p.bias_h_stride == 0 && !no_aff) ? align1k(2 * p.Cout * 4) : 0;
-    const int fixed = resident + align1k(kBarBytes) + union_bytes + rbox_bytes + sm_bytes + aff_bytes + 1024 /*alignment slack*/;
+    const int aff_bytes = ((BN <= 128 || p.k_blocks <= 4) && p.Cout <= 2048 && mode != 1 && p.bias_h_stride == 0) ? align1k(2 * p.Cout * 4) : 0;
+    const int fixed = align1k(kBarBytes) + union_bytes + rbox_bytes + sm_bytes + aff_bytes + 1024 /*alignment slack*/;
     int stages = (kSmemLimit - fixed) / stage_bytes;
     if (stages > kMaxStages) stages = kMaxStages;
     if (stages < 3) return -1;
-    static const int stage_cap = std::getenv("B200_STAGES") ? std::atoi(std::getenv("B200_STAGES")) : 0;  // experiments
-    if (stage_cap >= 2 && stages > stage_cap) stages = stage_cap;
     p.stages = stages;
-    p.off_ring = resident;
-    p.off_bar = resident + stages * stage_bytes;
+    p.off_bar = stages * stage_bytes;
     p.off_union = p.off_bar + align1k(kBarBytes);
     p.off_rbox = p.off_union + union_bytes;
     p.off_sm = p.off_rbox + rbox_bytes;
@@ -1264,7 +1210,7 @@ struct GemmJob {
     int K;         // reduction length = taps * Cin
 };
 
-static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, bool want_ws, cudaStream_t stream) {
+static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, cudaStream_t stream) {
     if (g_num_sms == 0) {
         int dev = 0;
         cudaGetDevice(&dev);
@@ -1281,51 +1227,30 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, bool want_ws, 
     const int ndot = p.dot_w != nullptr ? p.ndot : 0;
     auto divides = [&](int bn) { return Cout % bn == 0 && n_split % bn == 0 && (!two || seg2 % bn == 0); };
     int BN = 0, smem_bytes = -1;
-    bool ws = false;
-    if (want_ws && p.taps == 1 && ndot == 0 && mode == 0 && p.b_mode == 0) {
-        for (int bn : {128, 64}) {
-            if (!divides(bn) || Cout / bn > g_num_sms || p.k_blocks * bn * kBlockK * 2 > 128 * 1024) continue;
-            smem_bytes = plan_smem(p, bn, true, has_out, has_res, 0, 0);
-            if (smem_bytes > 0) {
-                BN = bn;
-                ws = true;
-                break;
-            }
-        }
-    }
     // TMA-staged epilogue?  Needs the warp's 32-row slab to be a {bw, bh} box and bf16 output / residual.
-    static const bool no_tma_up2 = std::getenv("B200_NO_TMA_UP2") != nullptr;
     const bool slab_is_box = p.BB == 1 && p.BW * p.BH == kBlockM && (p.BW % 32 == 0 || 32 % p.BW == 0) &&
                              (p.H == 1 || p.b_mode == 1 || p.H % p.BH == 0);
-    p.tma_epi = ((p.up2 && no_tma_up2) || p.res_f32 || p.out_f32 || !slab_is_box) ? 0 : 1;
+    p.tma_epi = (p.res_f32 || p.out_f32 || !slab_is_box) ? 0 : 1;
     p.share_box = 0;
-    if (!ws) {
-        static const bool no_share = std::getenv("B200_NO_SHARE_BOX") != nullptr;  // experiments
-        for (int bn : {256, 128, 64}) {
-            if (!divides(bn) || ((ndot != 0 || mode == 1) && bn != Cout)) continue;
-            // BN = 256 with a plain staged output: one 4 KB slot per warp instead of two buys a 4th ring stage,
-            // and the kernel is TMA-latency bound with three (measured: 2 -> 3 stages = +17..32 %)
-            const bool share = bn == 256 && p.tma_epi && has_out && !has_res && p.gap == nullptr && ndot == 0 &&
-                               mode == 0 && !p.up2 && !no_share;
-            // staging boxes exist only for the TMA epilogue (mode 2 keeps its transposition blocks)
-            const bool st_out = has_out && (p.tma_epi || mode == 2), st_res = has_res && p.tma_epi;
-            // BN = 128: pair two M tiles per iteration when there is enough work to keep every SM busy with pairs
-            static const bool no_pair = std::getenv("B200_NO_PAIR") != nullptr;  // A/B measurements
-            static const bool no_pair64 = std::getenv("B200_NO_PAIR64") != nullptr;
-            // (N = 64: only the 3x3 layers gain - 64->64 0.211 -> 0.158 ms; the 1x1 layers lose 5-9 %)
-            static const bool no_pair_dot = std::getenv("B200_NO_PAIR_DOT") != nullptr;
-            const bool pair = ((bn == 128 && (ndot == 0 || (ndot == 9 && !no_pair_dot))) ||
-                               (bn == 64 && ndot == 0 && p.k_blocks >= 8 && !no_pair64)) &&
-                              mode == 0 && p.a_batched && p.b_mode == 0 && !no_pair &&
-                              (p.m_tiles / 2) * (Cout / bn) >= g_num_sms;
-            smem_bytes = plan_smem(p, bn, false, st_out, st_res, ndot, mode, share, pair);
-            p.pair = (pair && smem_bytes > 0) ? 1 : 0;
-            if (pair && smem_bytes <= 0) smem_bytes = plan_smem(p, bn, false, st_out, st_res, ndot, mode, share, false);
-            if (smem_bytes > 0) {
-                BN = bn;
-                p.share_box = share ? 1 : 0;
-                break;
-            }
+    for (int bn : {256, 128, 64}) {
+        if (!divides(bn) || ((ndot != 0 || mode == 1) && bn != Cout)) continue;
+        // BN = 256 with a plain staged output: one 4 KB slot per warp instead of two buys a 4th ring stage,
+        // and the kernel is TMA-latency bound with three (measured: 2 -> 3 stages = +17..32 %)
+        const bool share = bn == 256 && p.tma_epi && has_out && !has_res && p.gap == nullptr && ndot == 0 &&
+                           mode == 0 && !p.up2;
+        // staging boxes exist only for the TMA epilogue (mode 2 keeps its transposition blocks)
+        const bool st_out = has_out && (p.tma_epi || mode == 2), st_res = has_res && p.tma_epi;
+        // BN = 128: pair two M tiles per iteration when there is enough work to keep every SM busy with pairs
+        // (N = 64: only the 3x3 layers gain - 64->64 0.211 -> 0.158 ms; the 1x1 layers lose 5-9 %)
+        const bool pair = ((bn == 128 && (ndot == 0 || ndot == 9)) || (bn == 64 && ndot == 0 && p.k_blocks >= 8)) &&
+                          mode == 0 && p.a_batched && p.b_mode == 0 && (p.m_tiles / 2) * (Cout / bn) >= g_num_sms;
+        smem_bytes = plan_smem(p, bn, st_out, st_res, ndot, mode, share, pair);
+        p.pair = (pair && smem_bytes > 0) ? 1 : 0;
+        if (pair && smem_bytes <= 0) smem_bytes = plan_smem(p, bn, st_out, st_res, ndot, mode, share, false);
+        if (smem_bytes > 0) {
+            BN = bn;
+            p.share_box = share ? 1 : 0;
+            break;
         }
     }
     if (BN == 0) return -13;
@@ -1402,33 +1327,15 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, bool want_ws, 
             return rc - 5000;
     }
     const int total = p.pair ? ((p.m_tiles + 1) / 2) * p.n_tiles : p.m_tiles * p.n_tiles;
-    int grid = total < g_num_sms ? total : g_num_sms;
-    if (ws) {  // every CTA keeps one N tile: the grid is a whole number of N-tile groups
-        const int groups = g_num_sms / p.n_tiles < p.m_tiles ? g_num_sms / p.n_tiles : p.m_tiles;
-        grid = groups * p.n_tiles;
-    }
+    const int grid = total < g_num_sms ? total : g_num_sms;
     const bool g = p.gap != nullptr;
     const int rm = p.res_mode;
-    if (ws) {
-        if (BN == 128)
-            return dispatch<128, true>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
-        return dispatch<64, true>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
-    }
-    if (BN == 256)
-        return dispatch<256, false>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
-    if (BN == 128)
-        return dispatch<128, false>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
-    return dispatch<64, false>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
+    if (BN == 256) return dispatch<256>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
+    if (BN == 128) return dispatch<128>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
+    return dispatch<64>(rm, g, ndot, mode, tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, stream);
 }
 
 }  // namespace b200
-
-extern "C" int b200_conv_gemm(const void* x, int x_ld, const void* w, const float* scale, const float* bias,
-                              const void* res, int res_ld, int res_mode, int act, void* out, int out_ld, int up2,
-                              float* gap, int B, int H, int W, int Cin, int Cout, int taps, void* stream) {
-    return b200_conv_gemm_ex(x, x_ld, w, scale, bias, res, res_ld, res_mode, act, out, out_ld, up2, gap, Cout, nullptr,
-                             0, 0, nullptr, 0, 0.f, nullptr, B, H, W, Cin, Cout, taps, 1, 1, stream);
-}
 
 static int conv_gemm_launch(const void* x, int x_ld, const void* w, const float* scale, const float* bias,
                             const void* res, int res_ld, int res_mode, int act, void* out, int out_ld, int up2,
@@ -1478,8 +1385,7 @@ static int conv_gemm_launch(const void* x, int x_ld, const void* w, const float*
         // Small ragged maps: a tile may span several cases (the 4th box dimension).  14 x 14 (ViT grid) as 9-row tiles
         // fills 196 of every 256 MMA rows; one image row of 9 consecutive cases per tile fills 126 of 128.  Pick the
         // (rows, cases) box with the best fill; plain stride-1 convolutions with the direct epilogue only.
-        static const bool no_multi = std::getenv("B200_NO_MULTICASE") != nullptr;  // A/B measurements
-        if (ragged && cs == 1 && !two && dot_w == nullptr && B > 1 && !no_multi) {
+        if (ragged && cs == 1 && !two && dot_w == nullptr && B > 1) {
             double best = static_cast<double>(Ho) * Wo / (p.tiles_h * 128.0);
             int best_bh = p.BH, best_bb = 1;
             for (int bh = 1; bh <= Ho && bh * Wo <= 128; ++bh) {
@@ -1548,10 +1454,6 @@ static int conv_gemm_launch(const void* x, int x_ld, const void* w, const float*
                    {out2_ld, static_cast<long long>(out2_ld) * Wo, static_cast<long long>(out2_ld) * Wo * Ho}};
     j.res = View4{res, {n_split, Wo, Ho, B},
                   {res_ld, static_cast<long long>(res_ld) * Wo, static_cast<long long>(res_ld) * Wo * Ho}};
-    // Measured on B200 (tools/kbench.py): the weight-stationary variant is slower than the streamed one for
-    // every layer of this model (it needs BN <= 128, i.e. twice the tiles and activation re-reads), so it
-    // is opt-in (B200_WS=1) until a 2-CTA / multicast version makes it pay.
-    static const bool want_ws = std::getenv("B200_WS") != nullptr;
     int mode = 0;
     if (drop.seg != 0) {
         if (dot_w != nullptr || up2 || res_mode == 2) return -19;  // dropout variants: plain / residual (+ channel sums)
@@ -1562,7 +1464,7 @@ static int conv_gemm_launch(const void* x, int x_ld, const void* w, const float*
         p.drop_seed_hi = static_cast<unsigned int>(drop.seed >> 32);
         p.drop_seg = drop.seg;
     }
-    return run_job(p, j, mode, mode == 0 && want_ws, static_cast<cudaStream_t>(stream));
+    return run_job(p, j, mode, static_cast<cudaStream_t>(stream));
 }
 extern "C" int b200_conv_gemm_ex(const void* x, int x_ld, const void* w, const float* scale, const float* bias,
                                  const void* res, int res_ld, int res_mode, int act, void* out, int out_ld, int up2,
@@ -1642,7 +1544,7 @@ static int linear_launch(const void* x, long long M, int K, const void* w, int N
         p.drop_seed_hi = static_cast<unsigned int>(drop.seed >> 32);
         p.drop_seg = drop.seg;
     }
-    return run_job(p, j, mode, false, static_cast<cudaStream_t>(stream));
+    return run_job(p, j, mode, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int b200_linear(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
@@ -1723,5 +1625,5 @@ extern "C" int b200_gemm_batched(const b200_gemm_desc* d, void* stream) {
                  {d->b_row_stride, d->b_head_stride, d->b_batch_stride}};
     j.out = View4{d->out, {d->N, d->M, d->heads, d->batch}, {d->out_row_stride, d->out_head_stride, d->out_batch_stride}};
     j.res = View4{d->res, {d->N, d->M, d->heads, d->batch}, {d->res_row_stride, d->res_head_stride, d->res_batch_stride}};
-    return run_job(p, j, d->mode, false, static_cast<cudaStream_t>(stream));
+    return run_job(p, j, d->mode, static_cast<cudaStream_t>(stream));
 }

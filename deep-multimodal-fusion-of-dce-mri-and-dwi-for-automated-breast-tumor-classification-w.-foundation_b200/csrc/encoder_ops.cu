@@ -674,14 +674,6 @@ extern "C" int b200_stem_mc(const float* x, int B, int C, int H, int W, int stri
                        n_mid, skip_out, mid_out, mod_attn, in_affine, z_lo, z_hi, in_table, L, d, stream);
 }
 
-extern "C" int b200_stem(const float* x, int B, int C, int H, int W, int stride, const float* plane_mean,
-                         const float* se_w1, const float* se_b1, const float* se_w2, const float* se_b2, int Cm,
-                         const float* wcat, const float* scale, const float* bias, int n_skip, int n_mid,
-                         void* skip_out, void* mid_out, float* mod_attn, void* stream) {
-    return b200_stem_ex(x, B, C, H, W, stride, plane_mean, se_w1, se_b1, se_w2, se_b2, Cm, wcat, scale, bias, n_skip, n_mid,
-                        skip_out, mid_out, mod_attn, nullptr, 0.f, 0.f, nullptr, 0, stream);
-}
-
 extern "C" int b200_se_gate(const float* gap_sum, int B, int C, int Cm, int npix, const float* w1t, const float* b1,
                             const float* w2t, const float* b2, float* gate, float* hidden, void* stream) {
     if (B < 0 || C <= 0 || Cm <= 0 || npix <= 0) return -1;

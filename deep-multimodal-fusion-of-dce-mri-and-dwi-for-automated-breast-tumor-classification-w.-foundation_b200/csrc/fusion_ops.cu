@@ -1,6 +1,6 @@
 // Late-fusion head (code/model_module.py:919-1000, FusionModel.forward) - the per-case
 // vector/token part and the elementwise mix.  The GEMM-shaped pieces (proj_in_*, mask
-// head `pre`, recon head, projector) run through b200_conv_gemm.
+// head `pre`, recon head, projector) run through b200_conv_gemm_ex.
 //
 //   fusion_tokens : adaptive 4x4 average pooling of a projected map into tokens (:903-917)
 //   fusion_core   : one CTA per case - gating softmax (:745-780, :952-956), multi-head

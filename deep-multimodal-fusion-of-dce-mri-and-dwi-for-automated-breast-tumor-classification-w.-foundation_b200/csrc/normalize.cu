@@ -850,13 +850,6 @@ extern "C" int b200_nyul_transform_ex(const float* x, float* out, int planes, in
                                    exact, nullptr, stream);
 }
 
-extern "C" int b200_nyul_transform(const float* x, float* out, int planes, int C, int n, int L,
-                                   const double* avg_landmarks, const double* standard_scale, const int* prev_index,
-                                   const double* gamma, float* plane_mean, void* stream) {
-    return b200_nyul_transform_ex(x, out, planes, C, n, L, avg_landmarks, standard_scale, prev_index, gamma, plane_mean,
-                                  0, stream);
-}
-
 extern "C" int b200_plane_mean(const float* x, int planes, int n, float* plane_mean, void* stream) {
     using namespace b200;
     if (planes < 0 || n <= 0) return -1;

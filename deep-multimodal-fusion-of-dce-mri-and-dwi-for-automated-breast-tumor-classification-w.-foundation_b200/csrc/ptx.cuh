@@ -64,14 +64,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     }
 }
 
-// ------------------------------------------- programmatic dependent launch --
-// A kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may start while its predecessor in the
-// stream is still draining: `griddep_wait` blocks until every prerequisite grid has completed and its writes are
-// visible (a no-op for a plain launch); `griddep_launch_dependents` lets the NEXT kernel's CTAs be scheduled as soon
-// as every CTA of this grid has issued it or exited.
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // --------------------------------------------------------------------- TMA --
 __device__ __forceinline__ void tma_prefetch_desc(const void* tmap) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tmap)) : "memory");

@@ -9,66 +9,6 @@ namespace b200 {
 
 constexpr int kStemTile = 8;                        // 8 x 8 output pixels per CTA
 constexpr int kStemPatch = kStemTile * 2 + 5;       // 21 x 21 input pixels feed them (7x7, stride 2)
-constexpr int kStem7Out = 64;
-
-// y[b, oy, ox, :] = relu(scale * sum_{c, ky, kx} gate[b, c] * x[b, c, 2 oy + ky - 3, 2 ox + kx - 3] * w[:, c, ky, kx] + bias)
-// x fp32 NCHW, y bf16 NHWC [B, H/2, W/2, 64].  256 threads = 64 pixels x 4 groups of 16 output channels; one input
-// channel at a time is staged (its 21 x 21 patch and its [49][64] weight slab, weights transposed on the host).
-__global__ void __launch_bounds__(256)
-conv7x7_s2_kernel(const float* __restrict__ x, const float* __restrict__ gate, int C, int H, int W,
-                  const float* __restrict__ wt,  // [C][49][64]
-                  const float* __restrict__ scale, const float* __restrict__ bias, __nv_bfloat16* __restrict__ y) {
-    __shared__ float s_patch[kStemPatch * kStemPatch];
-    __shared__ __align__(16) float s_w[49 * kStem7Out];
-    const int Ho = H / 2, Wo = W / 2;
-    const int b = blockIdx.z;
-    const int oy0 = blockIdx.y * kStemTile, ox0 = blockIdx.x * kStemTile;
-    const int tid = threadIdx.x;
-    const int pp = tid & 63, grp = tid >> 6;
-    const int py = pp >> 3, px = pp & 7;
-    float acc[16];
-#pragma unroll
-    for (int k = 0; k < 16; ++k) acc[k] = 0.f;
-    for (int c = 0; c < C; ++c) {
-        __syncthreads();
-        const float g = gate != nullptr ? gate[b * C + c] : 1.f;
-        const float* plane = x + (static_cast<size_t>(b) * C + c) * H * W;
-        for (int i = tid; i < kStemPatch * kStemPatch; i += 256) {
-            const int iy = oy0 * 2 - 3 + i / kStemPatch, ix = ox0 * 2 - 3 + i % kStemPatch;
-            s_patch[i] = (iy >= 0 && iy < H && ix >= 0 && ix < W) ? __ldg(plane + static_cast<size_t>(iy) * W + ix) * g : 0.f;
-        }
-        const float4* wsrc = reinterpret_cast<const float4*>(wt + static_cast<size_t>(c) * 49 * kStem7Out);
-        for (int i = tid; i < 49 * kStem7Out / 4; i += 256) reinterpret_cast<float4*>(s_w)[i] = __ldg(wsrc + i);
-        __syncthreads();
-#pragma unroll 1
-        for (int ky = 0; ky < 7; ++ky) {
-#pragma unroll
-            for (int kx = 0; kx < 7; ++kx) {
-                const float xv = s_patch[(py * 2 + ky) * kStemPatch + px * 2 + kx];
-                const float4* w4 = reinterpret_cast<const float4*>(s_w + (ky * 7 + kx) * kStem7Out + grp * 16);
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float4 wv = w4[q];
-                    acc[4 * q + 0] = fmaf(xv, wv.x, acc[4 * q + 0]);
-                    acc[4 * q + 1] = fmaf(xv, wv.y, acc[4 * q + 1]);
-                    acc[4 * q + 2] = fmaf(xv, wv.z, acc[4 * q + 2]);
-                    acc[4 * q + 3] = fmaf(xv, wv.w, acc[4 * q + 3]);
-                }
-            }
-        }
-    }
-    const int oy = oy0 + py, ox = ox0 + px;
-    if (oy >= Ho || ox >= Wo) return;
-    float o0[8], o1[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        o0[k] = fmaxf(fmaf(acc[k], scale[grp * 16 + k], bias[grp * 16 + k]), 0.f);
-        o1[k] = fmaxf(fmaf(acc[8 + k], scale[grp * 16 + 8 + k], bias[grp * 16 + 8 + k]), 0.f);
-    }
-    uint4* dst = reinterpret_cast<uint4*>(y + ((static_cast<size_t>(b) * Ho + oy) * Wo + ox) * kStem7Out + grp * 16);
-    dst[0] = pack_bf16x8(o0);
-    dst[1] = pack_bf16x8(o1);
-}
 
 // im2col of the 7x7 / stride-2 / padding-3 stem for the tensor-core route: row (b, oy, ox) of the bf16 patch matrix
 // holds gate[b, c] * x[b, c, 2 oy + ky - 3, 2 ox + kx - 3] at column c * 49 + ky * 7 + kx (Conv2d weight order),
@@ -156,18 +96,6 @@ __global__ void maxpool3x3_s2_kernel(const __nv_bfloat16* __restrict__ x, int H,
 }  // namespace b200
 
 using namespace b200;
-
-extern "C" int b200_conv7x7_s2(const float* x, const float* gate, int B, int C, int H, int W, const float* wt,
-                               const float* scale, const float* bias, void* y, void* stream) {
-    if (B < 0 || C <= 0 || H <= 0 || W <= 0 || H % 2 != 0 || W % 2 != 0 || B > 65535) return -1;
-    if (B == 0) return 0;
-    if (x == nullptr || wt == nullptr || scale == nullptr || bias == nullptr || y == nullptr) return -2;
-    if ((reinterpret_cast<uintptr_t>(wt) & 15) || (reinterpret_cast<uintptr_t>(y) & 15)) return -3;
-    const dim3 grid((W / 2 + kStemTile - 1) / kStemTile, (H / 2 + kStemTile - 1) / kStemTile, B);
-    conv7x7_s2_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, gate, C, H, W, wt, scale, bias,
-                                                                           static_cast<__nv_bfloat16*>(y));
-    return launch_status();
-}
 
 extern "C" int b200_maxpool3x3_s2(const void* x, int B, int H, int W, int C, void* y, void* stream) {
     if (B < 0 || H <= 0 || W <= 0 || H % 2 != 0 || W % 2 != 0 || C <= 0 || C % 8 != 0) return -1;

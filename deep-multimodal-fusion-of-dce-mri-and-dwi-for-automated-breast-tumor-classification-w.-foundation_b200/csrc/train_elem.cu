@@ -1036,7 +1036,7 @@ mask_attn_bwd_kernel(const float* __restrict__ mask, const float* __restrict__ d
 }
 
 // ---------------------------------------------------------------------------------------------- stem backward ----
-// Forward (b200_stem with every output channel in the un-activated segment): z[b,p,n] = sum_c wcat[n,c] x[b,c,s*p] gate[b,c].
+// Forward (b200_stem_ex with every output channel in the un-activated segment): z[b,p,n] = sum_c wcat[n,c] x[b,c,s*p] gate[b,c].
 // Backward from dz [B, npix, N] bf16:  dwcat[n,c] += gate[b,c] * sum_p dz[b,p,n] x[b,c,sp];
 //   dgate[b,c] = sum_p x[b,c,sp] * sum_n dz[b,p,n] wcat[n,c].
 // One CTA per case, 256-pixel tiles of x staged in shared memory (channels padded to CP).  Phase A: thread = pixel,

@@ -28,7 +28,6 @@ initialised unless a state dict (or a local ``pretrained_path``) is loaded.
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn as nn
@@ -40,7 +39,6 @@ __all__ = ["build_medical_backbone", "build_vit_dino_backbone", "build_radimagen
 
 VIT_NAMES = ("vit_base_patch16_224", "dino_vitbase16_pretrain", "dino_vitbase16_pretrained")
 RESNET_NAMES = ("resnet50", "radimagenet", "radimagenet_resnet50")
-_STEM_ON_TENSOR_CORES = os.environ.get("B200_RESNET_SIMT_STEM") is None
 
 
 class _FeatureInfo:
@@ -280,8 +278,7 @@ class B200ResNetBackbone(nn.Module):
         kp = (w.shape[1] * 49 + 63) // 64 * 64   # conv1 as a GEMM over zero-padded im2col rows (Conv2d weight order)
         wg = torch.zeros((64, kp), dtype=torch.bfloat16, device=dev)
         wg[:, :w.shape[1] * 49] = w.flatten(1).to(torch.bfloat16)
-        pk = {"stem": (w.permute(1, 2, 3, 0).reshape(w.shape[1], 49, 64).contiguous(), s0, b0),
-              "stem_gemm": (wg, kp), "layers": []}
+        pk = {"stem": (s0, b0), "stem_gemm": (wg, kp), "layers": []}
         for li in range(4):
             blocks = []
             for blk in getattr(self, f"layer{li + 1}"):
@@ -316,15 +313,12 @@ class B200ResNetBackbone(nn.Module):
         dev = x.device
         pk = self._packed(dev)
         B = x.shape[0]
-        if _STEM_ON_TENSOR_CORES:
-            # conv1 + bn1 + ReLU as one GEMM over the im2col rows (18.8 -> ~5 ms per 256-case step against the
-            # fp32 SIMT kernel, which stays available: B200_RESNET_SIMT_STEM=1)
-            wg, kp = pk["stem_gemm"]
-            cols = nat.im2col7x7_s2(x, gate, kp)
-            t = nat.linear(cols, wg, scale=pk["stem"][1], bias=pk["stem"][2], act=2).view(B, x.shape[2] // 2,
-                                                                                          x.shape[3] // 2, 64)
-        else:
-            t = nat.conv7x7_s2(x, gate, *pk["stem"])
+        # conv1 + bn1 + ReLU as one GEMM over the im2col rows (18.8 -> ~5 ms per 256-case step against the fp32 SIMT
+        # direct convolution it replaced)
+        wg, kp = pk["stem_gemm"]
+        cols = nat.im2col7x7_s2(x, gate, kp)
+        s0, b0 = pk["stem"]
+        t = nat.linear(cols, wg, scale=s0, bias=b0, act=2).view(B, x.shape[2] // 2, x.shape[3] // 2, 64)
         t = nat.maxpool3x3_s2(t)   # [B, H/4, W/4, 64]
         chans = [256, 512, 1024, 2048]
         # where does feature fi (position in the returned list) have to land?

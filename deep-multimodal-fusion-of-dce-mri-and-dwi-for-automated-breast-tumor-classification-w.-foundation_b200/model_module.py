@@ -26,8 +26,6 @@ from __future__ import annotations
 import math
 from dataclasses import dataclass
 
-import os
-
 import torch
 import torch.nn as nn
 from torch.nn import init
@@ -679,11 +677,6 @@ def _nchw(t):
     return t.permute(0, 3, 1, 2)
 
 
-# Residual of a block's tail conv folded into its contraction (see _packed); B200_NO_TAIL_CAT=1 restores the
-# residual-in-the-epilogue form for A/B measurements.
-_TAIL_CAT = os.environ.get("B200_NO_TAIL_CAT") is None
-
-
 def _staged_tiles(H, W):
     """True when the GEMM kernel tiles an H x W map into whole 128-pixel boxes (W divides 128 and the rows per
     tile divide H): only then can its epilogue stage tiles in shared memory, which the fused per-case channel
@@ -973,7 +966,7 @@ class ModelMaskHeadBackbone(_PackedWeightsMixin, nn.Module):
             # skip conv and first bottleneck conv read the same map: one GEMM, two output segments
             f = pk["fused_in"]
             st = pk.get("stride", 1)
-            if "tail_cat" in pk and _TAIL_CAT and pk["tail_cat"]["w"].shape[1] <= 512:
+            if "tail_cat" in pk and pk["tail_cat"]["w"].shape[1] <= 512:
                 # the skip segment lands in the upper channels of the tail GEMM's K-concatenated input
                 tc = pk["tail_cat"]
                 B, H, W, _ = x.shape

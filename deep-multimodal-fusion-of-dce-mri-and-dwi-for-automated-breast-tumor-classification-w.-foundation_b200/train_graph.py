@@ -4,8 +4,8 @@ The reference trains `ModelMaskHeadBackbone` through torch autograd (code/train.
 train-mode BatchNorm (batch statistics, running-statistics update), active nn.Dropout, every parameter receiving a
 gradient.  Here the same arithmetic is an explicit tape:
 
-* every tensor-core convolution = three launches of hand-written kernels - forward `b200_conv_gemm` on the bf16
-  packed weights, data gradient `b200_conv_gemm` on the flipped / transposed packing, weight gradient
+* every tensor-core convolution = three launches of hand-written kernels - forward `b200_conv_gemm_ex` on the bf16
+  packed weights, data gradient `b200_conv_gemm_ex` on the flipped / transposed packing, weight gradient
   `b200_conv_wgrad` (tcgen05 with MN-major operands straight from the NHWC maps; csrc/conv_wgrad.cu);
 * BatchNorm statistics / apply / backward, activations, residual adds, dropout (Philox, regenerated in the backward
   pass), squeeze-excite, the mask head and mask-guided attention, the 1-channel convolutions, the stem, the

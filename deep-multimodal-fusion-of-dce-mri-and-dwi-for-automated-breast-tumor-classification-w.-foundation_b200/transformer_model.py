@@ -6,7 +6,7 @@ pre-norm transformer stage (PatchEmbed :7-32, TokensToFeatureMap :34-52, Transfo
 TransformerStage :137-175).  Inside ModelMaskHeadBackbone.forward the stage is scheduled as one fused sequence
 (model_module._transformer_stage: packed weights cached, LayerScale + residual folded into the GEMM epilogues, fp32
 residual stream).  Called on their own, the modules run the same sm_100a kernels in eval mode - linears on
-b200_conv_gemm / b200_linear, LayerNorm on b200_layernorm, softmax(q k^T) v on b200_attention - with the reference's
+b200_conv_gemm_ex / b200_linear, LayerNorm on b200_layernorm, softmax(q k^T) v on b200_attention - with the reference's
 tensor conventions (tokens [B, N, C] fp32 in and out, maps NCHW).  CUDA only; train mode raises (the training path
 of the hybrid stage is not built).
 """
@@ -80,7 +80,7 @@ class PatchEmbed(nn.Module):
 
     def forward(self, x):
         """x [B, C, H, W] -> (tokens [B, N, E] fp32, (H/p, W/p)) (reference :26-32): the strided conv as an implicit
-        GEMM on b200_conv_gemm (taps = 4), LayerNorm on b200_layernorm."""
+        GEMM on b200_conv_gemm_ex (taps = 4), LayerNorm on b200_layernorm."""
         nat = _nat(self, "PatchEmbed", x)
         if self.proj.kernel_size != (2, 2) or self.proj.stride != (2, 2):
             raise NotImplementedError("only patch_size=2 (the reference default) is built")

@@ -29,7 +29,7 @@ extern "C" {
 int b200_abi_version(void);
 
 /*
- * Implicit-GEMM convolution (1x1 or 3x3/pad 1, stride 1) or linear layer with fused
+ * Implicit-GEMM convolution (1x1, 3x3 / padding 1 or 2x2 / stride 2) or linear layer with fused
  * epilogue, tcgen05/TMEM + TMA.  Replaces nn.Conv2d+BatchNorm2d(eval)+GELU(+residual)
  * stacks: code/model_module.py:259-269 (bottleneck), :276-280 (skip), :113-118
  * (ReconHead), :150 (MaskHeadResize.pre), :337-345 (Projector), :386-390
@@ -41,22 +41,12 @@ int b200_abi_version(void);
  *   scale, bias  fp32 [Cout] per-output-channel affine (folded BatchNorm or conv bias); NULL = 1 / 0
  *   res    optional residual map (bf16, res_ld); res_mode 0 none, 1 add before the
  *          activation, 2 add after it
- *   act    0 none, 1 exact (erf) GELU
+ *   act    0 none, 1 GELU, 2 ReLU
  *   out    bf16 map (out_ld), or NULL to skip the store; up2 != 0 replicates every pixel
  *          into a 2x2 block of a [B,2H,2W,out_ld] map (AdaptiveAvgPool2d to twice the
  *          size, model_module.py:534,707-710, commuted past the 1x1 projector)
  *   gap    optional fp32 [B,Cout]; the per-case sum over pixels of the epilogue result is
  *          ACCUMULATED into it (caller zeroes it)
- * taps may also be 4: a 2x2 kernel with stride 2 and no padding (PatchEmbed, code/transformer_model.py:18-23),
- * k = (ky*2+kx)*Cin + c; the output map is then [B,H/2,W/2,*].
- * Requires Cin % 64 == 0, Cout % 64 == 0, and for convolutions 128 % Wout == 0, Hout % (128/Wout) == 0.
- */
-int b200_conv_gemm(const void* x, int x_ld, const void* w, const float* scale, const float* bias,
-                   const void* res, int res_ld, int res_mode, int act, void* out, int out_ld, int up2,
-                   float* gap, int B, int H, int W, int Cin, int Cout, int taps, void* stream);
-
-/*
- * b200_conv_gemm with two extensions used to fuse neighbouring layers of the reference graph:
  *   n_split/out2/out2_ld/act2: output channels [n_split, Cout) are a second layer that reads the same
  *     input (e.g. a block's skip conv and first bottleneck conv, code/model_module.py:299 and :303) and
  *     go to out2 with their own activation flag (no residual / gap / up2 on either segment then);
@@ -67,11 +57,16 @@ int b200_conv_gemm(const void* x, int x_ld, const void* w, const float* scale, c
  *     (code/model_module.py:117), finished by b200_tapsum.  ndot = 1: a following 1x1, C -> 1 convolution
  *     (MaskHeadResize.out, code/model_module.py:187).  Requires Cout in {64,128,256} (one N tile), H > 1
  *     and out == NULL: the C-channel map never reaches HBM and is never rounded to bf16.
-  * `stride` (1 or 2) applies to taps 1 / 9: the strided 1x1 convs of a down-sampling ResNetLiteBlock
+ *     dot_w == NULL disables it.
+ * taps may also be 4: a 2x2 kernel with stride 2 and no padding (PatchEmbed, code/transformer_model.py:18-23),
+ * k = (ky*2+kx)*Cin + c; the output map is then [B,H/2,W/2,*].
+ * `stride` (1 or 2) applies to taps 1 / 9: the strided 1x1 convs of a down-sampling ResNetLiteBlock
  * (code/model_module.py:259-262, :276-280) and the 3x3 / stride-2 / padding-1 stacks of MaskHeadResize (:153-181);
  * H and W are the INPUT size, the output map is H/stride x W/stride.  `dilation` (>= 1, taps 9 only; padding =
  * dilation) serves the dilated layer3 / layer4 of the ResNet-50 backbones built with output_stride 8
- * (code/foundation_model.py:243-250).  `act`: 0 none, 1 GELU, 2 ReLU.
+ * (code/foundation_model.py:243-250).
+ * Requires Cin % 64 == 0, Cout % 64 == 0, and for convolutions Wout <= 128; up2 and gap also need
+ * 128 % Wout == 0 and Hout % (128/Wout) == 0.
  */
 int b200_conv_gemm_ex(const void* x, int x_ld, const void* w, const float* scale, const float* bias,
                       const void* res, int res_ld, int res_mode, int act, void* out, int out_ld, int up2,
@@ -178,7 +173,7 @@ int b200_vit_feature(const float* t, int B, int n_patch, int E, void* out, int o
 
 /*
  * nn.Linear on a token matrix (code/transformer_model.py:93, :95, :123, :125): out[M,N] = epilogue(x[M,K] w[N,K]^T)
- * with the b200_conv_gemm epilogue (scale, bias, GELU, residual).  The residual and / or the output may be
+ * with the b200_conv_gemm_ex epilogue (scale, bias, GELU, residual).  The residual and / or the output may be
  * fp32 row-major [M,N] (res_f32 / out_f32): x + gamma * (W y + b) then accumulates into an fp32 stream.
  */
 int b200_linear(const void* x, long long M, int K, const void* w, int N, const float* scale, const float* bias,
@@ -224,17 +219,11 @@ int b200_dwi_normalize_ex(const float* x, float* out, int planes, int C, int n, 
  *   prev_index int32 [L], gamma fp64 [L]: floor and fractional part of q/100*(n-1), the
  *   "linear" percentile rule of np.percentile (:100), computed on the host in float64.
  * Planes above 32 768 samples (224 x 224) take the radix-select kernel.
- */
-int b200_nyul_transform(const float* x, float* out, int planes, int C, int n, int L, const double* avg_landmarks,
-                        const double* standard_scale, const int* prev_index, const double* gamma,
-                        float* plane_mean, void* stream);
-
-/*
- * Same transform with the arithmetic mode chosen by the caller.  exact = 0 (what b200_nyul_transform runs): the two
- * chained np.interp maps are composed once per plane, in fp64, into one <= L-segment piece-wise linear table
- * (np.interp's tie / fill semantics folded in) and every sample costs an fp32 segment search plus one fp64 fma -
- * equal to numpy within 1 fp32 ulp, i.e. far inside the 1e-5 contract.  exact = 1: numpy's own operation order in
- * fp64 without FMA contraction, bit-identical to the reference on > 99.9 % of the samples, ~6x the instructions.
+ * exact selects the arithmetic.  exact = 0: the two chained np.interp maps are composed once per plane, in fp64, into
+ * one <= L-segment piece-wise linear table (np.interp's tie / fill semantics folded in) and every sample costs an fp32
+ * segment search plus one fp64 fma - equal to numpy within 1 fp32 ulp, i.e. far inside the 1e-5 contract.  exact = 1:
+ * numpy's own operation order in fp64 without FMA contraction, bit-identical to the reference on > 99.9 % of the
+ * samples, ~6x the instructions.
  */
 int b200_nyul_transform_ex(const float* x, float* out, int planes, int C, int n, int L, const double* avg_landmarks,
                            const double* standard_scale, const int* prev_index, const double* gamma,
@@ -259,24 +248,17 @@ int b200_plane_mean(const float* x, int planes, int n, float* plane_mean, void* 
  *   se_w1 [Cm,C], se_b1 [Cm], se_w2 [C,Cm], se_b2 [C] fp32, or se_w1 == NULL for no gate
  *   wcat [n_skip+n_mid, C] fp32, scale/bias [n_skip+n_mid] folded BatchNorm
  *   skip_out [B,H/s,W/s,n_skip] bf16, mid_out [B,H/s,W/s,n_mid] bf16, mod_attn [B,C] fp32
- */
-int b200_stem(const float* x, int B, int C, int H, int W, int stride, const float* plane_mean, const float* se_w1,
-              const float* se_b1, const float* se_w2, const float* se_b2, int Cm, const float* wcat,
-              const float* scale, const float* bias, int n_skip, int n_mid, void* skip_out, void* mid_out,
-              float* mod_attn, void* stream);
-
-/*
- * b200_stem with the per-channel normalisation FUSED INTO ITS OPERAND LOAD (north_star (1); the reference normalises
- * per sample on the CPU in SingleInputDataset.__getitem__, code/dataset.py:70-98): x is then the RAW input and exactly
+ * The per-channel normalisation can be FUSED INTO THE OPERAND LOAD (north_star (1); the reference normalises per
+ * sample on the CPU in SingleInputDataset.__getitem__, code/dataset.py:70-98): x is then the RAW input and exactly
  * one of
  *   in_affine [B*C][4] {mean, 1/std, scale, offset} from b200_dwi_normalize_ex(out = NULL) - DWINormalize
  *             (code/dataset.py:14-41): y = fma(clamp((x - mean) * (1/std), z_lo, z_hi), scale, offset); a skipped
  *             (zeroed) channel carries {0,0,0,0};
  *   in_table  [B*C][56] fp64 from b200_nyul_transform_ex2(out = NULL) - the composed NyulStandardizer table
  *             (code/preprocess_helpers.py:85-120): orig[16] | slope[16] | value[16] | up[16] (fp32)
- * is given (both NULL: x is already normalised, as b200_stem).  plane_mean must then be the per-plane mean of the
- * NORMALISED values, which both statistics kernels emit.  The normalised tensor never exists in HBM: the raw input is
- * read once by the statistics kernel and once (the stride-s pixels only) here.
+ * is given.  plane_mean must then be the per-plane mean of the NORMALISED values, which both statistics kernels emit.
+ * The normalised tensor never exists in HBM: the raw input is read once by the statistics kernel and once (the
+ * stride-s pixels only) here.  Both NULL: x is already normalised.
  */
 int b200_stem_ex(const float* x, int B, int C, int H, int W, int stride, const float* plane_mean, const float* se_w1,
                  const float* se_b1, const float* se_w2, const float* se_b2, int Cm, const float* wcat,
@@ -372,18 +354,14 @@ int b200_add_maps(const void* a, const void* b, long long n_elems, void* out, vo
 
 /*
  * ResNet-50 backbone stem (timm / torchvision `resnet50` as built by code/foundation_model.py:15-68, :220-312):
- *   b200_conv7x7_s2     conv1 (7x7, stride 2, padding 3) + folded bn1 + ReLU on the fp32 NCHW input, optionally
- *                       scaled per (case, channel) by the modality-attention gate; wt is the weight transposed to
- *                       [C][49][64]; y bf16 NHWC [B, H/2, W/2, 64]
  *   b200_maxpool3x3_s2  nn.MaxPool2d(3, 2, 1) on an NHWC bf16 map
- *   b200_im2col7x7_s2   (below) the stem as a GEMM operand
+ *   b200_im2col7x7_s2   conv1 (7x7, stride 2, padding 3) as a GEMM operand: bf16 patch matrix [B * H/2 * W/2, Kp]
+ *                       (column c*49 + ky*7 + kx, zero padded to Kp, a multiple of 64) of the fp32 NCHW input, scaled
+ *                       per (case, channel) by the modality-attention gate (nullable); conv1 + folded bn1 + ReLU is
+ *                       then one b200_linear call
  * The bottlenecks run on b200_conv_gemm_ex (act = 2, stride, dilation, residual).
  */
-int b200_conv7x7_s2(const float* x, const float* gate, int B, int C, int H, int W, const float* wt, const float* scale,
-                    const float* bias, void* y, void* stream);
 int b200_maxpool3x3_s2(const void* x, int B, int H, int W, int C, void* y, void* stream);
-/* The same stem for the tensor cores: bf16 patch matrix [B * H/2 * W/2, Kp] (column c*49 + ky*7 + kx, zero padded to
- * Kp, a multiple of 64), gate applied; conv1 + bn1 + ReLU is then one b200_linear call. */
 int b200_im2col7x7_s2(const float* x, const float* gate, int B, int C, int H, int W, int Kp, void* out, void* stream);
 
 /* compute_adc_map (code/preprocess_helpers.py:133-167): x [B, C, n] fp32 DWI stacks (n = H*W), bvals [C] on the
@@ -597,7 +575,7 @@ int b200_adamw_groups(float* p, const float* g, float* m, float* v, long long n,
 int b200_conv_wgrad(const void* dy, int dy_ld, const void* x, int x_ld, float* dw, int B, int H, int W, int Cin,
                     int Cout, int taps, void* stream);
 
-/* fp32 master weights [Cout, Cin, kh, kw] -> bf16 [Cout, taps*Cin] (forward operand of b200_conv_gemm) and / or
+/* fp32 master weights [Cout, Cin, kh, kw] -> bf16 [Cout, taps*Cin] (forward operand of b200_conv_gemm_ex) and / or
  * bf16 [Cin, taps*Cout] with flipped taps (operand of the data gradient: dX = conv(dY, w_dgrad)).  Either may be NULL. */
 int b200_pack_conv_weights(const float* w, int Cout, int Cin, int taps, void* w_fwd, void* w_dgrad, void* stream);
 
@@ -666,7 +644,7 @@ int b200_mask_attn_bwd(const float* mask, const float* dA, int B, int npix, int 
                        const float* gnb, const float* wb, const float* bb, float eps, float* dm, float* dwa, float* dgnw,
                        float* dgnb, float* dwb, float* dbb, void* stream);
 
-/* Backward of b200_stem run with every output channel un-activated (training: BatchNorm follows): from dz
+/* Backward of b200_stem_ex run with every output channel un-activated (training: BatchNorm follows): from dz
  * [B, npix, N] bf16 to dwcat [N, C] and the modality-attention gate gradient dgate [B, C]. */
 int b200_stem_bwd(const float* x, int B, int C, int H, int W, int stride, const float* gate, const void* dz, int N,
                   const float* wcat, float* dwcat, float* dgate, void* stream);

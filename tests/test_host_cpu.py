@@ -41,16 +41,18 @@ def test_library_exports_every_declared_symbol():
     assert lib.b200_abi_version() == nat.ABI_VERSION
 
 
-def test_invalid_arguments_are_rejected_without_a_gpu():
+def test_ex_entry_points_reject_invalid_arguments_without_a_gpu():
     import b200_native as nat
 
     lib = nat.lib()
     # negative return = invalid argument, nothing launched (no CUDA call is reached)
-    assert lib.b200_conv_gemm(None, 64, None, None, None, None, 0, 0, 0, None, 0, 0, None, 1, 32, 32, 64, 64, 1, None) < 0
+    assert lib.b200_conv_gemm_ex(None, 64, None, None, None, None, 0, 0, 0, None, 0, 0, None, 64, None, 0, 0, None, 0,
+                                 0.0, None, 1, 32, 32, 64, 64, 1, 1, 1, None) < 0
     assert lib.b200_dwi_normalize(None, None, 5, 4, 16, 1, -3.0, 3.0, None, None) < 0   # planes % C != 0
     assert lib.b200_dwi_normalize(None, None, 0, 4, 16, 1, -3.0, 3.0, None, None) == 0  # empty batch is a no-op
-    assert lib.b200_nyul_transform(None, None, 6, 6, 16, 40, None, None, None, None, None, None) < 0  # L too large
-    assert lib.b200_stem(None, 1, 64, 8, 8, 2, None, None, None, None, None, 0, None, None, None, 8, 8, None, None, None, None) < 0
+    assert lib.b200_nyul_transform_ex(None, None, 6, 6, 16, 40, None, None, None, None, None, 0, None) < 0  # L too large
+    assert lib.b200_stem_ex(None, 1, 64, 8, 8, 2, None, None, None, None, None, 0, None, None, None, 8, 8, None, None, None,
+                            None, 0.0, 0.0, None, 0, None) < 0
 
 
 def test_training_kernels_reject_out_of_range_arguments_without_a_gpu():

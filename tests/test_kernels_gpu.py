@@ -466,17 +466,23 @@ def test_flip_planes():
     assert torch.equal(nat.flip_planes(x, True, True), torch.flip(x, dims=[-1, -2]))
 
 
-def test_resnet_stem_kernels_and_dilated_relu_conv():
+def test_resnet_gemm_stem_and_dilated_relu_conv():
     g = torch.Generator(device="cpu").manual_seed(9)
     x = torch.rand(3, 6, 64, 80, generator=g).to(DEV)
     gate = (torch.rand(3, 6, generator=g) + 0.5).to(DEV)
     w = (torch.randn(64, 6, 7, 7, generator=g) / math.sqrt(6 * 49)).to(DEV)
     scale = (torch.rand(64, generator=g) + 0.5).to(DEV)
     bias = (torch.randn(64, generator=g) * 0.1).to(DEV)
-    y = nat.conv7x7_s2(x, gate, w.permute(1, 2, 3, 0).reshape(6, 49, 64).contiguous(), scale, bias)
-    ref = F.relu(F.conv2d(x * gate.view(3, 6, 1, 1), w, stride=2, padding=3) * scale.view(1, -1, 1, 1) +
+    # the stem as B200ResNetBackbone runs it: bf16 im2col rows (gate applied) and one GEMM with the folded BN + ReLU
+    kp = (6 * 49 + 63) // 64 * 64
+    wg = torch.zeros(64, kp, dtype=torch.bfloat16, device=DEV)
+    wg[:, :6 * 49] = w.flatten(1).bfloat16()
+    y = nat.linear(nat.im2col7x7_s2(x, gate, kp), wg, scale=scale, bias=bias, act=2).view(3, 32, 40, 64)
+    # reference on the bf16-rounded operands: only the accumulation order and the output rounding differ
+    xg = (x * gate.view(3, 6, 1, 1)).bfloat16().float()
+    ref = F.relu(F.conv2d(xg, w.bfloat16().float(), stride=2, padding=3) * scale.view(1, -1, 1, 1) +
                  bias.view(1, -1, 1, 1)).permute(0, 2, 3, 1)
-    assert tuple(y.shape) == (3, 32, 40, 64) and _rel(y, ref) < 5e-3
+    assert _rel(y, ref) < 5e-3
     p = nat.maxpool3x3_s2(y)
     refp = F.max_pool2d(y.float().permute(0, 3, 1, 2), 3, stride=2, padding=1).permute(0, 2, 3, 1)
     assert torch.equal(p.float(), refp)

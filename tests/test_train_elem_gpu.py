@@ -631,7 +631,7 @@ def test_mask_attn_bwd_vs_fp64(K, npix, bb):
                                                  (9, 16, 1, 17, 16, True), (16, 128, 1, 12, 23, True),
                                                  (17, 32, 2, 22, 40, False), (32, 256, 1, 16, 17, True)])
 def test_stem_bwd_vs_fp64(C, N, stride, H, W, gate):
-    """first layer backward (b200_stem, all outputs un-activated): z[b,p,n] = sum_c wcat[n,c] x[b,c,s p] gate[b,c];
+    """first layer backward (b200_stem_ex, all outputs un-activated): z[b,p,n] = sum_c wcat[n,c] x[b,c,s p] gate[b,c];
     dwcat += (accumulated), dgate += ; CP = 8 / 16 / 32 instantiations, pixel counts that are not a multiple of 256"""
     B = 2
     g = _g(C * 100 + N + stride)
