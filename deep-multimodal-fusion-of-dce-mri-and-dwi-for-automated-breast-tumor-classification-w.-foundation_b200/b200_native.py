@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # csrc/build.sh links the library at <repo>/lib/libb200fusion.so: a short path without the dots and dashes of the
 # package directory name, which is the path string dlopen sees.
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb200fusion.so")
-ABI_VERSION = 23
+ABI_VERSION = 24
 
 _lib = None
 

@@ -6,6 +6,7 @@
 // `qkv = Linear(E, 3E)(x).reshape(B, N, 3, heads, d)`, i.e. row (b, n) of the qkv buffer holds q | k | v, each
 // [heads, d] - exactly what the TMA boxes below pick apart.
 //
+// This kernel (attn_fused_kernel) serves N <= 256; attn_long_kernel below streams the keys for 256 < N <= 16384.
 // One work item = (case, head, 128-query tile); persistent CTAs, 160 threads:
 //   warp 4 (one elected lane)  TMA: Q box {64, 128} and K box {64, 256} per 64-wide slice of d (128-byte swizzle,
 //                              K-major operands), V box {64, 256} (the same rows, used MN-major: keys are the MMA's
@@ -49,8 +50,9 @@ struct AttnParams {
     int out_ld;
     float scale_log2;  // scale * log2(e)
     __nv_bfloat16* out;
-    // attention dropout (attn_fused_kernel<DH, true> only): probability (case b, head h, query row, key j) is dropped
-    // when word j % 4 of Philox4x32-7(seed; ((b * heads + h) * N + row) * 64 + j / 4) < drop_thresh
+    // attention dropout (DROP = true only): probability (case b, head h, query row, key j) is dropped when word j % 4
+    // of Philox4x32-7(seed; ((b * heads + h) * N + row) * 64 * ceil(N / 256) + j / 4) < drop_thresh (a 64-bit counter;
+    // the row stride is 64 for every N <= 256, so each row owns counters of its own at any N)
     unsigned int drop_thresh;
     float drop_scale;  // 1 / (1 - p), folded into the row's 1 / sum
     unsigned int drop_seed_lo, drop_seed_hi;
@@ -316,6 +318,259 @@ attn_fused_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// attn_long_kernel<DH, DROP>: the same contract for 256 < N <= kAtLongMaxN, with the keys streamed in 128-key tiles
+// through an online softmax.  One work item = (case, head, 128-query tile); persistent CTAs, one per SM, 192 threads:
+//   warp 4 (one lane)  TMA: Q box {64, 128} once per item; K and V of key tile j (rows j*128 .. j*128+127 of the case,
+//                      the same {64, 128} box) into ring stage j % 2.  Rows past N arrive as zeros (OOB fill).
+//   warp 5 (one lane)  allocates 512 TMEM columns: S buffers at columns 0 and 128, O at 256 .. 256+DH.
+//                      MMA 1: S[j % 2] = Q K_j^T, issued one tile ahead, so S_{j+1} is computed while the softmax
+//                      reads S_j.  MMA 2: O (+)= P_j V_j (V MN-major from its natural layout, as above).
+//   warps 0-3          one query row per thread: S_j -> 128 registers (read out of TMEM once), then P_j -> the one
+//                      swizzled K-major P buffer, fp32 row sum l; at the end of the item O * (1 / l) -> bf16 -> global.
+//
+// Ordering (mbarriers; "commit" = tcgen05.commit, which arrives once every earlier MMA of the issuing thread retired):
+//   q_full   TMA -> MMA (tx bytes)        q_empty   commit after the item's last MMA 1 -> TMA may load the next Q
+//   kv_full  TMA -> MMA (tx bytes)        kv_empty  commit after MMA 2 of the tile -> TMA may refill the stage
+//   s_full   commit after MMA 1 -> softmax            s_empty   128 arrivals once S_j is in registers -> MMA 1 of j+2
+//   p_full   128 arrivals: P_j stored (fence.proxy.async) and O rescaled (tcgen05.wait::st) -> MMA 2 of tile j
+//   o_full   commit after MMA 2 of tile j -> softmax: P free for P_{j+1}, O may be rescaled / read
+//   o_empty  128 arrivals once the item's O left TMEM -> first MMA 2 of the next item (which overwrites O)
+// Every softmax thread passes every wait, live rows or not, so no thread arrives on a barrier's next phase early.
+//
+// Online softmax with a lazy, conditionally moved reference m (log2 units, per row): m starts at the max of the first
+// key tile; a later tile moves it only when its max exceeds m by more than kAtRescaleLog2 (tau), and then l and the
+// row of O are scaled by 2^(m_old - m_new) (O through tcgen05.ld / st, after o_full of the previous tile).  Otherwise
+// the exponents stay <= 2^tau: harmless in fp32 l and bf16 P.  Scores rising slowly never pay for a rescale.
+//
+// Shared memory: Q KC x 16 KB + 2 stages x (K + V) KC x 16 KB + P 32 KB = 192 KB at d = 128, 112 KB at d = 64.  At
+// d = 64 one CTA per SM as well: two would need a single S buffer each (256 TMEM columns: S 128 + O 64), which
+// serialises MMA 1 behind the softmax; the launch asks for at least 116 KB so that two CTAs never share an SM (each
+// allocates 512 TMEM columns).
+constexpr int kAtLongThreads = 192;
+constexpr int kAtLongMaxN = 16384;   // a 128 x 128 token grid
+constexpr float kAtRescaleLog2 = 8.0f;
+constexpr int kAtLongMinSmem = 116 * 1024;
+
+template <int DH>
+struct AtLongSmem {
+    static constexpr int KC = DH / 64;
+    static constexpr int kTile = KC * kAtQBox;  // one 128-row box per 64-wide slice of d
+    static constexpr int kQ = 0, kK = kTile, kV = 3 * kTile, kP = 5 * kTile, kBars = 5 * kTile + 2 * kAtQBox;
+    static constexpr int kBytes = kBars + 128 /*barriers*/ + 1024 /*alignment slack*/;
+    static constexpr int kLaunch = kBytes > kAtLongMinSmem ? kBytes : kAtLongMinSmem;
+};
+
+template <int DH, bool DROP>
+__global__ void __launch_bounds__(kAtLongThreads, 1)
+attn_long_kernel(const __grid_constant__ CUtensorMap tm, const AttnParams p) {
+    using L = AtLongSmem<DH>;
+    constexpr int KC = L::KC;
+    extern __shared__ uint8_t smem_raw[];
+    uint8_t* smem = smem_raw + ((1024u - (static_cast<uint32_t>(__cvta_generic_to_shared(smem_raw)) & 1023u)) & 1023u);
+    uint8_t* const s_q = smem + L::kQ;
+    uint8_t* const s_k = smem + L::kK;  // stage s at s * kTile
+    uint8_t* const s_v = smem + L::kV;
+    uint8_t* const s_p = smem + L::kP;  // 2 x [128 rows x 128 B]: keys 0-63 | 64-127 of the tile
+    uint64_t* const bars = reinterpret_cast<uint64_t*>(smem + L::kBars);
+    uint64_t* const q_full = bars + 0;
+    uint64_t* const q_empty = bars + 1;
+    uint64_t* const kv_full = bars + 2;   // [2]
+    uint64_t* const kv_empty = bars + 4;  // [2]
+    uint64_t* const s_full = bars + 6;    // [2]
+    uint64_t* const s_empty = bars + 8;   // [2]
+    uint64_t* const p_full = bars + 10;
+    uint64_t* const o_full = bars + 11;
+    uint64_t* const o_empty = bars + 12;
+    uint32_t* const tmem_slot = reinterpret_cast<uint32_t*>(bars + 14);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int n_kt = (p.N + 127) >> 7;  // key tiles
+    if (threadIdx.x == 0) {
+        mbar_init(q_full, 1);
+        mbar_init(q_empty, 1);
+        for (int s = 0; s < 2; ++s) {
+            mbar_init(kv_full + s, 1);
+            mbar_init(kv_empty + s, 1);
+            mbar_init(s_full + s, 1);
+            mbar_init(s_empty + s, 128);
+        }
+        mbar_init(p_full, 128);
+        mbar_init(o_full, 1);
+        mbar_init(o_empty, 128);
+        fence_mbar_init();
+    }
+    if (warp == 5) tmem_alloc<512>(tmem_slot);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t tmem_o = tmem_base + 256;
+    const int E = p.heads * DH;
+
+    if (warp == 4) {
+        if (lane == 0) {
+            tma_prefetch_desc(&tm);
+            uint32_t t = 0, it = 0;
+            for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++it) {
+                const int qt = item % p.q_tiles;
+                const int h = (item / p.q_tiles) % p.heads;
+                const int b = item / (p.q_tiles * p.heads);
+                mbar_wait(q_empty, (it & 1u) ^ 1u);
+                mbar_arrive_expect_tx(q_full, L::kTile);
+#pragma unroll
+                for (int kc = 0; kc < KC; ++kc)
+                    tma_load_4d(s_q + kc * kAtQBox, &tm, q_full, h * DH + kc * 64, qt * 128, b, 0);
+                for (int j = 0; j < n_kt; ++j, ++t) {
+                    const int s = t & 1;
+                    mbar_wait(kv_empty + s, ((t >> 1) & 1u) ^ 1u);
+                    mbar_arrive_expect_tx(kv_full + s, 2 * L::kTile);
+#pragma unroll
+                    for (int kc = 0; kc < KC; ++kc) {
+                        tma_load_4d(s_k + s * L::kTile + kc * kAtQBox, &tm, kv_full + s, E + h * DH + kc * 64, j * 128, b, 0);
+                        tma_load_4d(s_v + s * L::kTile + kc * kAtQBox, &tm, kv_full + s, 2 * E + h * DH + kc * 64, j * 128,
+                                    b, 0);
+                    }
+                }
+            }
+        }
+    } else if (warp == 5) {
+        if (lane == 0) {
+            constexpr uint32_t idesc1 = umma_idesc_bf16(128, 128);
+            constexpr uint32_t idesc2 = umma_idesc_bf16(128, DH) | (1u << 16);  // B (= V) is MN-major
+            uint32_t t = 0, it = 0;
+            // MMA 1 of key tile j of the current item, the CTA's tile number tt
+            auto issue_s = [&](int j, uint32_t tt) {
+                const int s = tt & 1;
+                mbar_wait(kv_full + s, (tt >> 1) & 1u);
+                mbar_wait(s_empty + s, ((tt >> 1) & 1u) ^ 1u);
+                tc_fence_after();
+#pragma unroll
+                for (int kc = 0; kc < KC; ++kc) {
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) {
+                        const uint64_t da = umma_desc_sw128(smem_u32(s_q + kc * kAtQBox) + k * 32);
+                        const uint64_t db = umma_desc_sw128(smem_u32(s_k + s * L::kTile + kc * kAtQBox) + k * 32);
+                        umma_bf16(tmem_base + s * 128, da, db, idesc1, (kc | k) != 0 ? 1u : 0u);
+                    }
+                }
+                umma_commit(s_full + s);
+                if (j == n_kt - 1) umma_commit(q_empty);
+            };
+            for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++it) {
+                mbar_wait(q_full, it & 1u);
+                tc_fence_after();
+                issue_s(0, t);
+                for (int j = 0; j < n_kt; ++j, ++t) {
+                    if (j + 1 < n_kt) issue_s(j + 1, t + 1);
+                    if (j == 0) mbar_wait(o_empty, (it & 1u) ^ 1u);  // the previous item's O has left TMEM
+                    mbar_wait(p_full, t & 1u);
+                    tc_fence_after();
+                    const int s = t & 1;
+#pragma unroll
+                    for (int ks = 0; ks < 8; ++ks) {
+                        const uint64_t da = umma_desc_sw128(smem_u32(s_p + (ks >> 2) * kAtQBox) + (ks & 3) * 32);
+                        const uint64_t db = at_desc_mn_sw128(smem_u32(s_v + s * L::kTile) + ks * 2048, kAtQBox);
+                        umma_bf16(tmem_o, da, db, idesc2, (j | ks) != 0 ? 1u : 0u);
+                    }
+                    umma_commit(kv_empty + s);
+                    umma_commit(o_full);
+                }
+            }
+        }
+    } else {
+        const uint32_t lane_off = static_cast<uint32_t>(warp * 32) << 16;
+        const int r = warp * 32 + lane;  // row inside the query tile
+        const int swz = r & 7;
+        const unsigned long long ctr_stride = 64ull * ((p.N + 255) >> 8);
+        uint32_t t = 0, it = 0;
+        for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++it) {
+            const int qt = item % p.q_tiles;
+            const int h = (item / p.q_tiles) % p.heads;
+            const int b = item / (p.q_tiles * p.heads);
+            const int row = qt * 128 + r;
+            const bool warp_live = qt * 128 + warp * 32 < p.N;  // some row of this warp is a real query
+            unsigned long long ctr = 0;
+            if (DROP) ctr = ((static_cast<unsigned long long>(b) * p.heads + h) * p.N + row) * ctr_stride;
+            float m = 0.f, l = 0.f;
+            for (int j = 0; j < n_kt; ++j, ++t) {
+                const int s = t & 1;
+                uint32_t v[128];
+                mbar_wait(s_full + s, (t >> 1) & 1u);
+                tc_fence_after();
+                if (warp_live) {
+#pragma unroll
+                    for (int c = 0; c < 4; ++c)
+                        tmem_ld_32x32(tmem_base + lane_off + s * 128 + c * 32, *reinterpret_cast<uint32_t(*)[32]>(v + 32 * c));
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) tmem_ld_wait32(*reinterpret_cast<uint32_t(*)[32]>(v + 32 * c));
+                }
+                tc_fence_before();
+                mbar_arrive(s_empty + s);
+                const int valid = p.N - j * 128;
+                float mx = -3.0e38f;
+                if (warp_live) {
+                    float m4[4] = {-3.0e38f, -3.0e38f, -3.0e38f, -3.0e38f};
+#pragma unroll
+                    for (int i = 0; i < 128; ++i)
+                        if (i < valid) m4[i & 3] = fmaxf(m4[i & 3], __uint_as_float(v[i]));
+                    mx = fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])) * p.scale_log2;
+                }
+                if (j != 0) {
+                    mbar_wait(o_full, (t - 1) & 1u);  // MMA 2 of tile j-1 retired: P is free, O is final for j-1
+                    tc_fence_after();
+                }
+                if (warp_live) {
+                    if (j == 0) m = mx;
+                    const bool move = mx > m + kAtRescaleLog2;
+                    if (__any_sync(0xffffffffu, move)) {
+                        const float alpha = move ? ex2_approx(m - mx) : 1.0f;
+                        if (move) m = mx;
+                        l *= alpha;
+#pragma unroll
+                        for (int c = 0; c < DH / 32; ++c) {
+                            uint32_t o[32];
+                            tmem_ld_32x32(tmem_o + lane_off + c * 32, o);
+                            tmem_ld_wait32(o);
+#pragma unroll
+                            for (int i = 0; i < 32; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
+                            tmem_st_32x32(tmem_o + lane_off + c * 32, o);
+                        }
+                        tmem_st_wait();
+                    }
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) {
+                        uint8_t* const dst = s_p + (c >> 1) * kAtQBox + r * 128;
+                        const uint32_t(&vc)[32] = *reinterpret_cast<const uint32_t(*)[32]>(v + 32 * c);
+                        const unsigned long long cc = ctr + j * 32 + c * 8;
+                        if (valid >= 128)
+                            l += softmax_chunk<false, DROP>(vc, p.scale_log2, -m, 32, dst, (c & 1) * 4, swz, p, cc);
+                        else
+                            l += softmax_chunk<true, DROP>(vc, p.scale_log2, -m, valid - c * 32, dst, (c & 1) * 4, swz, p,
+                                                           cc);
+                    }
+                }
+                fence_proxy_async_smem();  // P (generic-proxy stores) -> visible to the MMA's async-proxy reads
+                tc_fence_before();
+                mbar_arrive(p_full);
+            }
+            mbar_wait(o_full, (t - 1) & 1u);  // the item's last MMA 2 retired
+            tc_fence_after();
+            if (warp_live)
+                store_rows<DH>(tmem_o + lane_off, p.out + (static_cast<long long>(b) * p.N + row) * p.out_ld + h * DH,
+                               row < p.N, (DROP ? p.drop_scale : 1.0f) / l);
+            tc_fence_before();
+            mbar_arrive(o_empty);
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 5) {
+        tc_fence_after();
+        tmem_dealloc<512>(tmem_base);
+    }
+}
+
 
 typedef CUresult (*AtEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -365,10 +620,26 @@ static int at_launch(const CUtensorMap& tmQ, const CUtensorMap& tmKV, const Attn
     return static_cast<int>(cudaGetLastError());
 }
 
+template <int DH, bool DROP>
+static int at_long_launch(const CUtensorMap& tm, const AttnParams& p, int num_sms, cudaStream_t s) {
+    constexpr int smem = AtLongSmem<DH>::kLaunch;
+    static bool configured = false;
+    if (!configured) {
+        cudaError_t e = cudaFuncSetAttribute(attn_long_kernel<DH, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return static_cast<int>(e);
+        configured = true;
+    }
+    const int grid = num_sms < p.n_items ? num_sms : p.n_items;
+    attn_long_kernel<DH, DROP><<<grid, kAtLongThreads, smem, s>>>(tm, p);
+    return static_cast<int>(cudaGetLastError());
+}
+
 // Argument checks, tensor maps and launch of b200_attention / b200_attention_mc (drop_p in [0, 1); 0 = no dropout).
+// N <= 256 runs attn_fused_kernel (one score tile per item), 256 < N <= kAtLongMaxN attn_long_kernel.
 static int attention_run(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh, float scale,
                          float drop_p, unsigned long long drop_seed, void* stream) {
-    if (B < 0 || N <= 0 || N > 256 || heads <= 0 || (dh != 64 && dh != 128)) return -1;
+    if (B < 0 || N <= 0 || N > kAtLongMaxN || heads <= 0 || (dh != 64 && dh != 128)) return -1;
+    if (N > 256 && static_cast<long long>(B) * heads * ((N + 127) / 128) > 0x7fffffffLL) return -1;  // items are ints
     if (B == 0) return 0;
     if (qkv == nullptr || out == nullptr) return -2;
     const int E = heads * dh;
@@ -386,7 +657,7 @@ static int attention_run(const void* qkv, int qkv_ld, void* out, int out_ld, int
     CUtensorMap tmQ, tmKV;
     int rc;
     if ((rc = at_encode_map(enc, &tmQ, qkv, 3 * E, qkv_ld, N, B, 128)) != 0) return rc - 1000;
-    if ((rc = at_encode_map(enc, &tmKV, qkv, 3 * E, qkv_ld, N, B, 256)) != 0) return rc - 2000;
+    if (N <= 256 && (rc = at_encode_map(enc, &tmKV, qkv, 3 * E, qkv_ld, N, B, 256)) != 0) return rc - 2000;
     AttnParams p{};
     p.N = N;
     p.heads = heads;
@@ -404,8 +675,12 @@ static int attention_run(const void* qkv, int qkv_ld, void* out, int out_ld, int
         p.drop_scale = 1.0f / (1.0f - drop_p);
         p.drop_seed_lo = static_cast<unsigned int>(drop_seed);
         p.drop_seed_hi = static_cast<unsigned int>(drop_seed >> 32);
+        if (N > 256)
+            return dh == 64 ? at_long_launch<64, true>(tmQ, p, num_sms, s) : at_long_launch<128, true>(tmQ, p, num_sms, s);
         return dh == 64 ? at_launch<64, true>(tmQ, tmKV, p, num_sms, s) : at_launch<128, true>(tmQ, tmKV, p, num_sms, s);
     }
+    if (N > 256)
+        return dh == 64 ? at_long_launch<64, false>(tmQ, p, num_sms, s) : at_long_launch<128, false>(tmQ, p, num_sms, s);
     return dh == 64 ? at_launch<64, false>(tmQ, tmKV, p, num_sms, s) : at_launch<128, false>(tmQ, tmKV, p, num_sms, s);
 }
 

@@ -154,8 +154,6 @@ class B200ViTBackbone(nn.Module):
         g = self.grid
         n = g * g          # patch tokens
         N = n + 1          # + cls
-        if N > 256:
-            raise NotImplementedError("more than 256 tokens per image (b200_attention holds one 256-key score tile)")
         dev = x.device
         pk = self._packed(dev)
         K0 = C * P * P

@@ -46,8 +46,8 @@ def _tokens_bf16(x):
 def _attention_tokens(nat, at, h, B, N):
     """h [B*N, C] bf16 (already normalised) -> proj(softmax(q k^T / sqrt d) v) [B*N, C] bf16 (reference :98-116)."""
     C = at.embed_dim
-    if at.head_dim not in (64, 128) or N > 256:
-        raise NotImplementedError("b200_attention: head_dim 64 or 128, at most 256 tokens")
+    if at.head_dim not in (64, 128):
+        raise NotImplementedError("b200_attention: head_dim 64 or 128")
     bqkv = _f(at.qkv.bias) if at.qkv.bias is not None else torch.zeros(3 * C, device=h.device)
     qkv = nat.linear(h, _w(at.qkv.weight), bias=bqkv)
     o = torch.empty((B * N, C), dtype=torch.bfloat16, device=h.device)

@@ -96,9 +96,12 @@ int b200_conv_gemm_mc(const void* x, int x_ld, const void* w, const float* scale
  * MultiHeadSelfAttention.forward between its qkv and proj layers (code/transformer_model.py:101-112; attn_drop is
  * identity in eval mode) and the timm ViT-B/16 attention of the backbone (code/foundation_model.py:371-431).
  * One launch, no score / probability buffer in HBM: S in TMEM -> softmax in registers -> P in shared memory -> P V.
- * bf16 in / out, fp32 accumulation and softmax.  N <= 256 tokens, dh in {64, 128}; qkv_ld >= 3*heads*dh, out_ld >=
- * heads*dh, both multiples of 8 elements, 16-byte aligned bases.  Returns 0, -1 unsupported shape, -2 null pointer,
- * -3 leading dimensions, -5 alignment.
+ * N <= 256 holds a query tile's whole score row in TMEM; 256 < N <= 16384 streams the keys in 128-key tiles through an
+ * online softmax.  bf16 in / out, fp32 accumulation and softmax.  1 <= N <= 16384 tokens, dh in {64, 128}; qkv_ld >=
+ * 3*heads*dh, out_ld >= heads*dh, both multiples of 8 elements, 16-byte aligned bases.  Returns 0 (also for B == 0,
+ * nothing launched), -1 unsupported shape (N or dh out of range, B < 0, heads <= 0, or more than 2^31 - 1 work items
+ * B * heads * ceil(N / 128) at N > 256), -2 null pointer, -3 leading dimensions, -5 alignment, -8 / -9 / <= -1000
+ * driver or tensor-map errors, > 0 a CUDA error of the launch.  Nothing is launched when the result is < 0.
  */
 int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh, float scale,
                    void* stream);
@@ -106,7 +109,8 @@ int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, in
 /*
  * b200_attention with the attention dropout of MC-dropout inference (nn.Dropout(drop_p) in train mode on the softmax
  * probabilities, code/transformer_model.py:109-116): probability (b, h, n, j) is kept when word j % 4 of
- * Philox4x32-7(drop_seed; ((b * heads + h) * N + n) * 64 + j / 4) >= drop_p * 2^32, else it is 0; the row sums are
+ * Philox4x32-7(drop_seed; ((b * heads + h) * N + n) * 64 * ceil(N / 256) + j / 4) >= drop_p * 2^32, else it is 0
+ * (the counter is a 64-bit integer; for N <= 256 its row stride is 64); the row sums are
  * those of the undropped softmax and the kept probabilities are scaled by 1 / (1 - drop_p).  The decision depends
  * only on the seed and the indices.  drop_p == 0 runs b200_attention.  Returns -19 unless 0 <= drop_p < 1 (nothing
  * launched), else as b200_attention.
