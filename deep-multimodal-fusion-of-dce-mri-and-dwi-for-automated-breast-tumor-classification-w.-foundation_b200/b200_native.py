@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # csrc/build.sh links the library at <repo>/lib/libb200fusion.so: a short path without the dots and dashes of the
 # package directory name, which is the path string dlopen sees.
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb200fusion.so")
-ABI_VERSION = 24
+ABI_VERSION = 25
 
 _lib = None
 
@@ -41,26 +41,6 @@ class FusionWeights(C.Structure):
         ("up_coef", C.c_void_p),
         ("se_w1t", C.c_void_p), ("se_b1", C.c_void_p), ("se_w2t", C.c_void_p), ("se_b2", C.c_void_p),
         ("cls_w", C.c_void_p), ("cls_b", C.c_void_p),
-    ]
-
-
-class GemmDesc(C.Structure):
-    """Mirror of `struct b200_gemm_desc` (include/b200_fusion.h)."""
-
-    _fields_ = [
-        ("M", C.c_int), ("N", C.c_int), ("K", C.c_int), ("heads", C.c_int), ("batch", C.c_int),
-        ("a", C.c_void_p), ("a_row_stride", C.c_longlong), ("a_head_stride", C.c_longlong),
-        ("a_batch_stride", C.c_longlong), ("a_shared", C.c_int),
-        ("b", C.c_void_p), ("b_row_stride", C.c_longlong), ("b_head_stride", C.c_longlong),
-        ("b_batch_stride", C.c_longlong),
-        ("out", C.c_void_p), ("out_row_stride", C.c_longlong), ("out_head_stride", C.c_longlong),
-        ("out_batch_stride", C.c_longlong),
-        ("res", C.c_void_p), ("res_row_stride", C.c_longlong), ("res_head_stride", C.c_longlong),
-        ("res_batch_stride", C.c_longlong),
-        ("res_mode", C.c_int), ("act", C.c_int),
-        ("scale", C.c_void_p), ("bias", C.c_void_p), ("vec_h_stride", C.c_int),
-        ("rowscale", C.c_void_p), ("mode", C.c_int), ("alpha", C.c_float), ("n_valid", C.c_int),
-        ("rowsum_inv", C.c_void_p), ("b_rows", C.c_int),
     ]
 
 
@@ -102,7 +82,6 @@ SIGNATURES = {
     "b200_resize_aa_c1": [_P, _I, _I, _I, _P, _I, _I, _P],
     "b200_mask_attention": [_P, _I, _I, _I, _P, _P, _P, _P, _P, _F, _P, _P],
     "b200_tapsum": [_P, _I, _I, _I, _P, _P, _P],
-    "b200_gemm_batched": [C.POINTER(GemmDesc), _P],
     "b200_layernorm": [_P, _I, _LL, _I, _P, _P, _F, _P, _I, _P],
     "b200_patchify": [_P, _P, _I, _I, _I, _I, _I, _P, _P],
     "b200_vit_tokens": [_P, _P, _P, _I, _I, _I, _P, _P],
@@ -121,7 +100,6 @@ SIGNATURES = {
     "b200_se_gate": [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P],
     "b200_scale_map": [_P, _P, _I, _I, _I, _P, _P, _P, _P],
     "b200_conv3x3_c1": [_P, _I, _I, _I, _I, _P, _P, _P, _P],
-    "b200_mask_tail": [_P, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P, _F, _P, _P],
     "b200_lift_c1": [_P, _LL, _I, _P, _P, _P, _P, _P],
     "b200_cls_head": [_P, _P, _I, _I, _I, _I, _P, _P, _I, _P, _P, _P],
     "b200_channel_sums": [_P, _I, _I, _I, _I, _P, _P],
@@ -320,24 +298,6 @@ def conv_gemm(x, w, *, taps, scale=None, bias=None, res=None, res_mode=0, act=0,
     else:
         _call("b200_conv_gemm_ex", key, *args, _stream())
     return out if n_split is None else (out, out2)
-
-
-def gemm_batched(*, M, N, K, heads, batch, a, a_strides, b, b_strides, out, out_strides, a_shared=False, res=None,
-                 res_strides=(0, 0, 0), res_mode=0, act=0, scale=None, bias=None, vec_h_stride=0, rowscale=None,
-                 mode=0, alpha=1.0, n_valid=0, rowsum_inv=None, b_rows=0):
-    """Batched K-major GEMM (see b200_gemm_batched).  a / b / out / res are data pointers (ints) so that views
-    with channel offsets can be passed; strides are (row, head, batch) in elements."""
-    d = GemmDesc()
-    d.M, d.N, d.K, d.heads, d.batch = M, N, K, heads, batch
-    d.a, (d.a_row_stride, d.a_head_stride, d.a_batch_stride), d.a_shared = a, a_strides, int(a_shared)
-    d.b, (d.b_row_stride, d.b_head_stride, d.b_batch_stride) = b, b_strides
-    d.out, (d.out_row_stride, d.out_head_stride, d.out_batch_stride) = out, out_strides
-    d.res, (d.res_row_stride, d.res_head_stride, d.res_batch_stride) = res, res_strides
-    d.res_mode, d.act = res_mode, act
-    d.scale, d.bias, d.vec_h_stride = _ptr(scale), _ptr(bias), vec_h_stride
-    d.rowscale, d.mode, d.alpha, d.n_valid, d.rowsum_inv = _ptr(rowscale), mode, float(alpha), n_valid, _ptr(rowsum_inv)
-    d.b_rows = b_rows
-    _call("b200_gemm_batched", (batch, heads, M, K, N, mode), C.byref(d), _stream())
 
 
 def layernorm(x, w, b, eps, out=None, out_dtype=torch.bfloat16):
@@ -556,16 +516,6 @@ def conv3x3_c1(x, w, bias, out):
     B, H, W, C_ = x.shape
     _call("b200_conv3x3_c1", None, _ptr(x), B, H, W, C_, _ptr(w), _ptr(bias), _ptr(out), _stream())
     return out
-
-
-def mask_tail(pre, w_out, b_out, mask_pred, attn_params=None, attn=None):
-    B, H, W, Cm = pre.shape
-    if attn_params is None:
-        hc, wa, gw, gb, wb, bb, eps = 0, None, None, None, None, None, 0.0
-    else:
-        hc, wa, gw, gb, wb, bb, eps = attn_params
-    _call("b200_mask_tail", None, _ptr(pre), B, H * W, Cm, _ptr(w_out), _ptr(b_out), _ptr(mask_pred), hc, _ptr(wa),
-                                _ptr(gw), _ptr(gb), _ptr(wb), _ptr(bb), float(eps), _ptr(attn), _stream())
 
 
 def mask_attention(mask, attn_params, attn):

@@ -84,19 +84,12 @@ struct ConvGemmParams {
     int a_box_bytes;       // bytes one A box really delivers (BW*BH rows x 128 B; < 16 KB when BW*BH < 128)
     int cstride;           // convolution stride
     int dil;               // dilation of the 3x3 taps (1 = dense) (1, or 2 for the 2x2 / stride-2 patch embedding: taps == 4)
-    int a_batched;         // 0: the A operand is shared by every (h, b) (weights on the A side)
-    int b_mode;            // 0: B operand = 2-D weights [N, K]; 1: 4-D batched {K, N, H, B}
-    int bias_h_stride;     // scale / bias index = n + h * bias_h_stride (per-head vectors in batched GEMMs)
-    const float* rowscale; // optional per-row multiplier [B, H, W] applied before scale / bias (1 / softmax sum)
-    float* rowsum_inv;     // MODE 1: receives 1 / sum_j exp(...) per row, [B, H, W]
-    float alpha;           // MODE 1: logits = alpha * acc
-    int n_valid;           // MODE 1: number of real columns (keys); the rest are masked out
     int res_f32, out_f32;  // residual / output are fp32 row-major (transformer residual stream); direct path
     int stages;            // operand ring depth
     int obuf2;             // output staging double-buffered per epilogue warp (tile i+1 is staged while the TMA store of
                            // tile i still reads its boxes); 0: one set of boxes, the store is waited for at the next tile
     int pair;              // BN = 128: two M tiles per CTA iteration share one weight slab (conv_gemm_kernel<..., PAIR>)
-    int off_bar, off_union, off_rbox, off_sm;  // shared-memory plan (bytes from the 1 KB-aligned base)
+    int off_bar, off_union, off_rbox;  // shared-memory plan (bytes from the 1 KB-aligned base)
     int off_aff;           // >= 0: [scale Cout | bias Cout] parked in shared memory once per CTA (BN <= 128 launches);
                            // -1: they are read from global memory per chunk
 };
@@ -164,10 +157,8 @@ __device__ __forceinline__ void dropout_chunk(float (&v)[kChunk], long long pix,
 // Epilogue features are compile-time so that the per-element instruction stream carries no flag tests:
 //   RES  0 none, 1 residual added before the activation, 2 after it
 //   GAP  per-case channel sums          NDOT 0, or 1 / 9 fused per-pixel dot products (no map store)
-//   MODE 0 standard; 1 row softmax numerator: out = exp(alpha*acc - rowmax) as bf16, 1/rowsum to rowsum_inv
-//        (the whole row lives in one N tile; the division is deferred to the consumer GEMM's rowscale);
-//        2 fp32 residual / output (b200_linear); 3 MC dropout after the activation; 4 = 2 with MC dropout before the
-//        residual add (b200_linear_mc)
+//   MODE 0 standard; 2 fp32 residual / output (b200_linear); 3 MC dropout after the activation; 4 = 2 with MC
+//        dropout before the residual add (b200_linear_mc)
 //   PAIR (BN = 128 only): a CTA works on TWO consecutive M tiles of the same N tile at once - 256 x 128 outputs: per
 //        64-deep k-block the weight slab is loaded once and feeds two MMAs (one per M tile, each with its own TMEM
 //        accumulator), so a stage moves 48 KB for 2 x (128 x 128 x 64) MACs instead of 64 KB.  128 x 128 tiles were
@@ -225,7 +216,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         }
         for (int s = 0; s < kAcc; ++s) {
             mbar_init(&tfull[s], 1);
-            mbar_init(&tempty[s], MODE == 1 ? kNumEpiWarps / 2 : kNumEpiWarps);  // mode 1: one warp set per stage
+            mbar_init(&tempty[s], kNumEpiWarps);
         }
         for (int s = 0; s < 2 * kNumEpiWarps; ++s) mbar_init(&resbar[s], 1);
         fence_mbar_init();
@@ -269,12 +260,10 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     mbar_wait(&empty[stage], phase ^ 1);
                     mbar_arrive_expect_tx(&full[stage], p.a_box_bytes * (has2 ? 2 : 1) + T::kBBytes);
                     uint8_t* dst = sRing + stage * kStageBytes;
-                    if (p.a_batched) tma_load_4d(dst, &tmA, &full[stage], c0, p.cstride * w0 + dx, p.cstride * h0 + dy, b);
-                    else tma_load_4d(dst, &tmA, &full[stage], c0, w0, 0, 0);
+                    tma_load_4d(dst, &tmA, &full[stage], c0, p.cstride * w0 + dx, p.cstride * h0 + dy, b);
                     if (has2) tma_load_4d(dst + kABytes, &tmA, &full[stage], c0, p.cstride * w1 + dx, p.cstride * h1 + dy, b1);
                     constexpr int kBOff = PAIR ? 2 * kABytes : kABytes;
-                    if (p.b_mode == 0) tma_load_2d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN);
-                    else tma_load_4d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN, h0, b);
+                    tma_load_2d(dst + kBOff, &tmB, &full[stage], kb * kBlockK, n_tile * BN);
                     if (++stage == stages) {
                         stage = 0;
                         phase ^= 1;
@@ -328,125 +317,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 }
             }
         }
-    } else if (MODE == 1 && warp >= kEpiWarp0) {
-        // Softmax-numerator epilogue (Q.K^T): out = bf16(exp(alpha * acc - rowmax)) over the n_valid real columns,
-        // zeros beyond, and 1 / rowsum per row.  The MMA side of these launches is tiny (K = head_dim), so the
-        // epilogue is the whole cost: each accumulator stage belongs to ONE set of four warps (one per TMEM lane
-        // quadrant), a warp owns complete rows - no row max / row sum exchange between warps, no named barriers -
-        // and the two sets work on consecutive tiles concurrently.  A warp's four 64-column output boxes rotate
-        // through its two 4 KB staging slots.
-        const int ew = warp - kEpiWarp0;
-        const int q = warp & 3;
-        const int set = ew >> 2;  // accumulator stage this warp serves
-        uint8_t* const obuf = s_union + ew * T::kWarpBoxBytes;
-        const int swz = ((lane * T::kRowBytes) >> 7) & (T::kRowBytes / 16 - 1);
-        const int row_off = lane * T::kRowBytes;
-        const float k2 = p.alpha * 1.4426950408889634f;  // exp(x) = exp2(x * log2 e)
-        constexpr int kChunks = BN / kChunk;             // 8 chunks of 32 columns
-        constexpr int kChunksPerBox = T::kBoxCols / kChunk;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        int tile = blockIdx.x;
-        for (int it = 0; it < n_iters; ++it, tile += gridDim.x) {
-            if (acc == set) {
-                const int m_tile = fd_div(p.fd_ntiles, tile);
-                int tw0, th0, b;
-                tile_whb(p, m_tile, tw0, th0, b);
-                const int w0 = tw0 * p.BW, h0 = th0 * p.BH;
-                const int slab_w = w0 + (q * 32) % p.BW, slab_h = h0 + (q * 32) / p.BW;
-                const int trow = q * 32 + lane;
-                const int pw = w0 + trow % p.BW, ph = h0 + trow / p.BW;
-                const bool valid = pw < p.W && ph < p.H;
-                const long long pix = (static_cast<long long>(b) * p.H + ph) * p.W + pw;
-                if (lane == 0) tma_store_wait_read<0>();  // the previous tile's boxes have left the staging slots
-                __syncwarp();
-                mbar_wait(&tfull[acc], acc_phase);
-                tc_fence_after();
-                const uint32_t tm_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN;
-                // pass 1: row maximum of the raw accumulator over the valid columns (alpha > 0 scales it afterwards)
-                float m = -INFINITY;
-#pragma unroll
-                for (int ch = 0; ch < kChunks; ch += 2) {
-                    const int c0 = ch * kChunk;
-                    if (c0 >= p.n_valid) break;  // warp-uniform
-                    uint32_t ra[kChunk], rb[kChunk];
-                    tmem_ld_32x32(tm_row + c0, ra);
-                    tmem_ld_32x32(tm_row + c0 + kChunk, rb);
-                    tmem_ld_wait();
-                    if (c0 + 2 * kChunk <= p.n_valid) {
-#pragma unroll
-                        for (int j = 0; j < kChunk; ++j)
-                            m = fmaxf(m, fmaxf(__uint_as_float(ra[j]), __uint_as_float(rb[j])));
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < kChunk; ++j) {
-                            if (c0 + j < p.n_valid) m = fmaxf(m, __uint_as_float(ra[j]));
-                            if (c0 + kChunk + j < p.n_valid) m = fmaxf(m, __uint_as_float(rb[j]));
-                        }
-                    }
-                }
-                const float row_max2 = m * k2;
-                // pass 2: numerators, bf16 rounding, row sum, staged stores
-                float row_sum = 0.f;
-#pragma unroll
-                for (int ch = 0; ch < kChunks; ++ch) {
-                    const int n0 = ch * kChunk;
-                    const int bx = ch / kChunksPerBox;
-                    uint8_t* const slot = obuf + (bx & 1) * T::kBoxBytes;
-                    const int c16 = (ch % kChunksPerBox) * (kChunk / 8);
-                    uint4 o[4];
-                    if (n0 < p.n_valid) {  // warp-uniform
-                        uint32_t r[kChunk];
-                        tmem_ld_32x32(tm_row + n0, r);
-                        tmem_ld_wait();
-                        const bool all_real = n0 + kChunk <= p.n_valid;
-                        uint32_t hb[kChunk / 2];
-#pragma unroll
-                        for (int j = 0; j < kChunk; j += 2) {
-                            float e0 = ex2_approx(fmaf(__uint_as_float(r[j]), k2, -row_max2));
-                            float e1 = ex2_approx(fmaf(__uint_as_float(r[j + 1]), k2, -row_max2));
-                            if (!all_real) {
-                                if (n0 + j >= p.n_valid) e0 = 0.f;
-                                if (n0 + j + 1 >= p.n_valid) e1 = 0.f;
-                            }
-                            // round to bf16 first: the row sum must match what the P.V GEMM will read
-                            const __nv_bfloat162 h2 = __floats2bfloat162_rn(e0, e1);
-                            hb[j / 2] = *reinterpret_cast<const uint32_t*>(&h2);
-                            row_sum += __uint_as_float(hb[j / 2] << 16) + __uint_as_float(hb[j / 2] & 0xffff0000u);
-                        }
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) o[j] = make_uint4(hb[4 * j], hb[4 * j + 1], hb[4 * j + 2], hb[4 * j + 3]);
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) o[j] = make_uint4(0u, 0u, 0u, 0u);
-                    }
-                    if (ch % kChunksPerBox == 0 && bx >= 2) {  // the slot still holds box bx - 2: wait for its TMA read
-                        if (lane == 0) tma_store_wait_read<1>();
-                        __syncwarp();
-                    }
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-                        *reinterpret_cast<uint4*>(slot + row_off + (((c16 + j) ^ swz) << 4)) = o[j];
-                    if (ch % kChunksPerBox == kChunksPerBox - 1) {  // box complete
-                        if (ch == kChunks - 1) {  // last TMEM read of the tile is done: release the accumulator stage
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) mbar_arrive(&tempty[acc]);
-                        }
-                        fence_proxy_async_smem();
-                        __syncwarp();
-                        if (lane == 0) {
-                            tma_store_4d(&tmOut, slot, bx * T::kBoxCols, slab_w, slab_h, b);
-                            tma_store_commit();
-                        }
-                    }
-                }
-                if (valid) p.rowsum_inv[pix] = 1.0f / row_sum;
-            }
-            acc ^= 1;
-            if (acc == 0) acc_phase ^= 1;
-        }
-        if (lane == 0) tma_store_wait_all<0>();
     } else if (warp >= kEpiWarp0) {
         const int ew = warp - kEpiWarp0;
         const int q = warp & 3;    // TMEM lane quadrant this warp may read (rows q*32 .. q*32+31 of the tile)
@@ -479,7 +349,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         // ([scale Cout | bias Cout] fp32): per 32-column chunk every lane needs the same 32 + 32 floats, which cost 16
         // LDG.128 + 32 descriptor moves (R2UR) per chunk and lane when read from global memory - 15 % of the instructions
         // of a BN = 64 tile (profiles/r2_ncu_full.csv, capture r2_k64).  BN <= 128 launches only (the host plans it).
-        float* const s_aff = (MODE != 1 && p.off_aff >= 0) ? reinterpret_cast<float*>(smem + p.off_aff) : nullptr;
+        float* const s_aff = p.off_aff >= 0 ? reinterpret_cast<float*>(smem + p.off_aff) : nullptr;
         if (s_aff != nullptr) {
             const int et = threadIdx.x - kEpiWarp0 * 32;  // 0 .. 255 over the epilogue warps
             for (int i = et; i < p.Cout / 4; i += kNumEpiWarps * 32) {
@@ -576,40 +446,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             mbar_wait(&tfull[acc], acc_phase);
             tc_fence_after();
             const uint32_t tm_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN + colw0;
-            const int vec_off = h0 * p.bias_h_stride;  // per-head scale / bias vectors (0 for convolutions)
-            const float row_mul = (MODE == 0 && p.rowscale != nullptr && valid) ? p.rowscale[pix] : 1.f;
-            float row_max2 = 0.f;  // MODE 1: row maximum of the logits, in log2 units
-            float* const s_sm = reinterpret_cast<float*>(smem + p.off_sm);  // [2 acc][2 halves][128] max, then sums
-            if (MODE == 1) {
-                // row maximum over the valid columns, on the raw accumulator (alpha > 0 scales it afterwards);
-                // two 32-column TMEM loads in flight per wait, chunks past n_valid are not read at all
-                float m = -INFINITY;
-#pragma unroll
-                for (int ch = 0; ch < T::kChunksPerWarp; ch += 2) {
-                    const int c0 = colw0 + ch * kChunk;
-                    if (c0 >= p.n_valid) break;  // warp-uniform
-                    uint32_t ra[kChunk], rb[kChunk];
-                    tmem_ld_32x32(tm_row + ch * kChunk, ra);
-                    tmem_ld_32x32(tm_row + (ch + 1) * kChunk, rb);
-                    tmem_ld_wait();
-                    if (c0 + 2 * kChunk <= p.n_valid) {
-#pragma unroll
-                        for (int j = 0; j < kChunk; ++j)
-                            m = fmaxf(m, fmaxf(__uint_as_float(ra[j]), __uint_as_float(rb[j])));
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < kChunk; ++j) {
-                            if (c0 + j < p.n_valid) m = fmaxf(m, __uint_as_float(ra[j]));
-                            if (c0 + kChunk + j < p.n_valid) m = fmaxf(m, __uint_as_float(rb[j]));
-                        }
-                    }
-                }
-                m *= p.alpha * 1.4426950408889634f;
-                s_sm[(acc * 2 + half) * kBlockM + trow] = m;
-                asm volatile("bar.sync 2, 256;" ::: "memory");
-                row_max2 = fmaxf(m, s_sm[(acc * 2 + (half ^ 1)) * kBlockM + trow]);
-            }
-            float row_sum = 0.f;
 #pragma unroll
             for (int ch = 0; ch < T::kChunksPerWarp; ++ch) {
                 const int n0 = nbase + ch * kChunk;
@@ -630,52 +466,27 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 tmem_ld_wait();
                 float v[kChunk];
                 float2* const v2 = reinterpret_cast<float2*>(v);
-                if (MODE == 1) {
-                    // softmax numerator: logits = alpha * acc (columns >= n_valid masked), e = exp(logit - rowmax)
-                    const float k2 = p.alpha * 1.4426950408889634f;  // work in log2 units: exp(x) = exp2(x*log2 e)
-                    const bool all_real = n0 + kChunk <= p.n_valid;  // warp-uniform
+                if (s_aff != nullptr) {
+                    const float4* s4 = reinterpret_cast<const float4*>(s_aff + n0);
+                    const float4* b4 = reinterpret_cast<const float4*>(s_aff + p.Cout + n0);
 #pragma unroll
-                    for (int j = 0; j < kChunk; j += 2) {
-                        float e0 = ex2_approx(fmaf(__uint_as_float(r[j]), k2, -row_max2));
-                        float e1 = ex2_approx(fmaf(__uint_as_float(r[j + 1]), k2, -row_max2));
-                        if (!all_real) {
-                            if (n0 + j >= p.n_valid) e0 = 0.f;
-                            if (n0 + j + 1 >= p.n_valid) e1 = 0.f;
-                        }
-                        // round to bf16 first: the row sum must match what the P.V GEMM will read
-                        const __nv_bfloat162 h2 = __floats2bfloat162_rn(e0, e1);
-                        const uint32_t hb = *reinterpret_cast<const uint32_t*>(&h2);
-                        v[j] = __uint_as_float(hb << 16);
-                        v[j + 1] = __uint_as_float(hb & 0xffff0000u);
-                        row_sum += v[j] + v[j + 1];
+                    for (int j = 0; j < kChunk / 4; ++j) {
+                        const float4 s = s4[j], t = b4[j];
+                        v2[2 * j + 0] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 0]), __uint_as_float(r[4 * j + 1])),
+                                                   make_float2(s.x, s.y), make_float2(t.x, t.y));
+                        v2[2 * j + 1] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3])),
+                                                   make_float2(s.z, s.w), make_float2(t.z, t.w));
                     }
                 } else {
-                    if (p.rowscale != nullptr) {
+                    const float4* s4 = reinterpret_cast<const float4*>(p.scale + n0);
+                    const float4* b4 = reinterpret_cast<const float4*>(p.bias + n0);
 #pragma unroll
-                        for (int j = 0; j < kChunk; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) * row_mul);
-                    }
-                    if (s_aff != nullptr) {
-                        const float4* s4 = reinterpret_cast<const float4*>(s_aff + n0);
-                        const float4* b4 = reinterpret_cast<const float4*>(s_aff + p.Cout + n0);
-#pragma unroll
-                        for (int j = 0; j < kChunk / 4; ++j) {
-                            const float4 s = s4[j], t = b4[j];
-                            v2[2 * j + 0] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 0]), __uint_as_float(r[4 * j + 1])),
-                                                       make_float2(s.x, s.y), make_float2(t.x, t.y));
-                            v2[2 * j + 1] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3])),
-                                                       make_float2(s.z, s.w), make_float2(t.z, t.w));
-                        }
-                    } else {
-                        const float4* s4 = reinterpret_cast<const float4*>(p.scale + n0 + vec_off);
-                        const float4* b4 = reinterpret_cast<const float4*>(p.bias + n0 + vec_off);
-#pragma unroll
-                        for (int j = 0; j < kChunk / 4; ++j) {
-                            const float4 s = __ldg(s4 + j), t = __ldg(b4 + j);
-                            v2[2 * j + 0] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 0]), __uint_as_float(r[4 * j + 1])),
-                                                       make_float2(s.x, s.y), make_float2(t.x, t.y));
-                            v2[2 * j + 1] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3])),
-                                                       make_float2(s.z, s.w), make_float2(t.z, t.w));
-                        }
+                    for (int j = 0; j < kChunk / 4; ++j) {
+                        const float4 s = __ldg(s4 + j), t = __ldg(b4 + j);
+                        v2[2 * j + 0] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 0]), __uint_as_float(r[4 * j + 1])),
+                                                   make_float2(s.x, s.y), make_float2(t.x, t.y));
+                        v2[2 * j + 1] = __ffma2_rn(make_float2(__uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3])),
+                                                   make_float2(s.z, s.w), make_float2(t.z, t.w));
                     }
                 }
                 // box / chunk position of these 32 columns inside the warp's staged boxes
@@ -917,13 +728,6 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&tempty[acc]);
-            if (MODE == 1) {
-                float* const s_sum = s_sm + 4 * kBlockM;
-                s_sum[(acc * 2 + half) * kBlockM + trow] = row_sum;
-                asm volatile("bar.sync 2, 256;" ::: "memory");
-                if (half == 0 && valid)
-                    p.rowsum_inv[pix] = 1.0f / (row_sum + s_sum[(acc * 2 + 1) * kBlockM + trow]);
-            }
             if (!DOT && tma_epi && out_ptr != nullptr) {
                 // one TMA store per staged box: full 64/128-byte row segments, rows past the end are clipped
                 fence_proxy_async_smem();
@@ -1047,12 +851,6 @@ static int dispatch(int res_mode, bool gap, int ndot, int mode, const CUtensorMa
                     const ConvGemmParams& p, int smem_bytes, int grid, cudaStream_t s) {
 #define B200_GO(RES, GAP, DOT, MODE) \
     return launch<BN, RES, GAP, DOT, MODE>(tmA, tmB, tmOut, tmOut2, tmRes, p, smem_bytes, grid, s)
-    if (mode == 1) {
-        if constexpr (BN == 256) {
-            if (res_mode == 0 && !gap && ndot == 0) B200_GO(0, false, 0, 1);
-        }
-        return -14;
-    }
     if (mode == 3) {  // MC-dropout epilogue (plain / residual, with or without channel sums)
         if (ndot == 0) {
             if (res_mode == 0 && gap) B200_GO(0, true, 0, 3);
@@ -1158,9 +956,8 @@ static int plan_smem(ConvGemmParams& p, int BN, bool has_out, bool has_res, int 
     }
     const int union_bytes = align1k(ndot ? dot_bytes : (has_out ? out_stage : 0));
     const int rbox_bytes = has_res ? align1k(box_all) : 0;
-    const int sm_bytes = mode == 1 ? align1k(8 * kBlockM * 4) : 0;  // row max / row sum exchange
-    const int aff_bytes = ((BN <= 128 || p.k_blocks <= 4) && p.Cout <= 2048 && mode != 1 && p.bias_h_stride == 0) ? align1k(2 * p.Cout * 4) : 0;
-    const int fixed = align1k(kBarBytes) + union_bytes + rbox_bytes + sm_bytes + aff_bytes + 1024 /*alignment slack*/;
+    const int aff_bytes = ((BN <= 128 || p.k_blocks <= 4) && p.Cout <= 2048) ? align1k(2 * p.Cout * 4) : 0;
+    const int fixed = align1k(kBarBytes) + union_bytes + rbox_bytes + aff_bytes + 1024 /*alignment slack*/;
     int stages = (kSmemLimit - fixed) / stage_bytes;
     if (stages > kMaxStages) stages = kMaxStages;
     if (stages < 3) return -1;
@@ -1168,8 +965,7 @@ static int plan_smem(ConvGemmParams& p, int BN, bool has_out, bool has_res, int 
     p.off_bar = stages * stage_bytes;
     p.off_union = p.off_bar + align1k(kBarBytes);
     p.off_rbox = p.off_union + union_bytes;
-    p.off_sm = p.off_rbox + rbox_bytes;
-    p.off_aff = aff_bytes ? p.off_sm + sm_bytes : -1;
+    p.off_aff = aff_bytes ? p.off_rbox + rbox_bytes : -1;
     return fixed + stages * stage_bytes;
 }
 
@@ -1203,9 +999,8 @@ static int encode_view(EncodeTiledFn encode, CUtensorMap* tm, const View4& v, co
 
 // Everything the two C entry points hand to the common launcher.
 struct GemmJob {
-    View4 a;       // {K, W, H, B}: K-major rows of the A operand (activations, or weights when !a_batched)
-    View4 b4;      // batched B operand {K, N, H, B} (b_mode 1)
-    const void* w; // 2-D weights [N, K] (b_mode 0)
+    View4 a;       // {K, W, H, B}: K-major rows of the A operand (the activations)
+    const void* w; // 2-D weights [N, K]
     View4 out, out2, res;  // {cols, W', H', B}
     int K;         // reduction length = taps * Cin
 };
@@ -1229,11 +1024,11 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, cudaStream_t s
     int BN = 0, smem_bytes = -1;
     // TMA-staged epilogue?  Needs the warp's 32-row slab to be a {bw, bh} box and bf16 output / residual.
     const bool slab_is_box = p.BB == 1 && p.BW * p.BH == kBlockM && (p.BW % 32 == 0 || 32 % p.BW == 0) &&
-                             (p.H == 1 || p.b_mode == 1 || p.H % p.BH == 0);
+                             (p.H == 1 || p.H % p.BH == 0);
     p.tma_epi = (p.res_f32 || p.out_f32 || !slab_is_box) ? 0 : 1;
     p.share_box = 0;
     for (int bn : {256, 128, 64}) {
-        if (!divides(bn) || ((ndot != 0 || mode == 1) && bn != Cout)) continue;
+        if (!divides(bn) || (ndot != 0 && bn != Cout)) continue;
         // BN = 256 with a plain staged output: one 4 KB slot per warp instead of two buys a 4th ring stage,
         // and the kernel is TMA-latency bound with three (measured: 2 -> 3 stages = +17..32 %)
         const bool share = bn == 256 && p.tma_epi && has_out && !has_res && p.gap == nullptr && ndot == 0 &&
@@ -1243,7 +1038,7 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, cudaStream_t s
         // BN = 128: pair two M tiles per iteration when there is enough work to keep every SM busy with pairs
         // (N = 64: only the 3x3 layers gain - 64->64 0.211 -> 0.158 ms; the 1x1 layers lose 5-9 %)
         const bool pair = ((bn == 128 && (ndot == 0 || ndot == 9)) || (bn == 64 && ndot == 0 && p.k_blocks >= 8)) &&
-                          mode == 0 && p.a_batched && p.b_mode == 0 && (p.m_tiles / 2) * (Cout / bn) >= g_num_sms;
+                          mode == 0 && (p.m_tiles / 2) * (Cout / bn) >= g_num_sms;
         smem_bytes = plan_smem(p, bn, st_out, st_res, ndot, mode, share, pair);
         p.pair = (pair && smem_bytes > 0) ? 1 : 0;
         if (pair && smem_bytes <= 0) smem_bytes = plan_smem(p, bn, st_out, st_res, ndot, mode, share, false);
@@ -1287,7 +1082,7 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, cudaStream_t s
                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B)) != 0)
             return rc - 1000;
     }
-    if (p.b_mode == 0) {
+    {
         const cuuint64_t dims[2] = {static_cast<cuuint64_t>(j.K), static_cast<cuuint64_t>(Cout)};
         const cuuint64_t strides[1] = {static_cast<cuuint64_t>(j.K) * 2};
         const cuuint32_t box[2] = {64, static_cast<cuuint32_t>(BN)};
@@ -1296,12 +1091,6 @@ static int run_job(ConvGemmParams& p, const GemmJob& j, int mode, cudaStream_t s
                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return -200 - static_cast<int>(r);
-    } else {
-        const int box[4] = {64, BN, 1, 1};
-        const int estr[4] = {1, 1, 1, 1};
-        if ((rc = encode_view(encode, &tmB, j.b4, box, estr, CU_TENSOR_MAP_SWIZZLE_128B,
-                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B)) != 0)
-            return rc - 2000;
     }
     // Staged (TMA) epilogue: per epilogue warp one {cw columns, bw, bh} box = its 32 rows x BN/2 columns
     // (two boxes when BN = 256), swizzled by the row width.  The 2x2-replicating store walks a
@@ -1419,11 +1208,6 @@ static int conv_gemm_launch(const void* x, int x_ld, const void* w, const float*
     p.k_blocks = taps * p.kc;
     p.cstride = cs;
     p.dil = dilation;
-    p.a_batched = 1;
-    p.b_mode = 0;
-    p.bias_h_stride = 0;
-    p.rowscale = nullptr;
-    p.rowsum_inv = nullptr;
     p.scale = scale;
     p.bias = bias;
     p.res = static_cast<const __nv_bfloat16*>(res);
@@ -1517,8 +1301,6 @@ static int linear_launch(const void* x, long long M, int K, const void* w, int N
     p.taps = 1;
     p.k_blocks = p.kc;
     p.cstride = 1;
-    p.a_batched = 1;
-    p.b_mode = 0;
     p.scale = scale;
     p.bias = bias;
     p.res = static_cast<const __nv_bfloat16*>(res);
@@ -1569,61 +1351,4 @@ extern "C" int b200_linear_mc(const void* x, long long M, int K, const void* w, 
     d.seg = 1;
     return linear_launch(x, M, K, w, N, scale, bias, res, res_f32, res_mode == 1 ? 2 : res_mode, act, out, out_f32, d,
                          stream);
-}
-
-extern "C" int b200_gemm_batched(const b200_gemm_desc* d, void* stream) {
-    using namespace b200;
-    if (d == nullptr || d->a == nullptr || d->b == nullptr) return -1;
-    if (d->M <= 0 || d->N <= 0 || d->K <= 0 || d->heads <= 0 || d->batch <= 0) return -1;
-    if (d->K % 8 != 0 || d->N % 64 != 0) return -2;  // K tail handled by TMA zero fill, rows by clipping
-    if (d->mode != 0 && d->mode != 1) return -2;
-    if (d->mode == 1 && (d->N != 256 || d->rowsum_inv == nullptr || d->out == nullptr || !(d->alpha > 0.f))) return -3;
-    if (d->res_mode != 0 && d->res == nullptr) return -4;
-    ConvGemmParams p{};
-    p.BB = 1;
-    p.B = d->batch;
-    p.H = d->heads;
-    p.W = d->M;
-    p.BW = 128;
-    p.BH = 1;
-    p.tiles_w = (d->M + 127) / 128;
-    p.tiles_h = d->heads;
-    p.Cout = d->N;
-    p.n_split = d->N;
-    p.m_tiles = d->batch * p.tiles_w * p.tiles_h;
-    p.kc = 0;  // unused when taps == 1 (tap = kb / kc is never evaluated with kc = k_blocks)
-    p.taps = 1;
-    p.k_blocks = (d->K + 63) / 64;
-    p.kc = p.k_blocks;
-    p.cstride = 1;
-    p.a_batched = d->a_shared ? 0 : 1;
-    p.b_mode = 1;
-    p.bias_h_stride = d->vec_h_stride;
-    p.rowscale = d->rowscale;
-    p.rowsum_inv = d->rowsum_inv;
-    p.alpha = d->alpha;
-    p.n_valid = d->n_valid > 0 ? d->n_valid : d->N;
-    p.scale = d->scale;
-    p.bias = d->bias;
-    p.res = static_cast<const __nv_bfloat16*>(d->res);
-    p.res_ld = static_cast<int>(d->res_row_stride);
-    p.res_mode = d->res_mode;
-    p.act = d->act;
-    p.out = static_cast<__nv_bfloat16*>(d->out);
-    p.out_ld = static_cast<int>(d->out_row_stride);
-    p.up2 = 0;
-    p.gap = nullptr;
-    p.out2 = nullptr;
-    p.dot_w = nullptr;
-    p.ndot = 0;
-    GemmJob j{};
-    j.K = d->K;
-    if (d->a_shared) j.a = View4{d->a, {d->K, d->M, 1, 1}, {d->a_row_stride, 0, 0}};
-    else j.a = View4{d->a, {d->K, d->M, d->heads, d->batch}, {d->a_row_stride, d->a_head_stride, d->a_batch_stride}};
-    // b_rows < N: the missing rows of the B operand are zero-filled by the TMA (ragged key / token counts)
-    j.b4 = View4{d->b, {d->K, d->b_rows > 0 ? d->b_rows : d->N, d->heads, d->batch},
-                 {d->b_row_stride, d->b_head_stride, d->b_batch_stride}};
-    j.out = View4{d->out, {d->N, d->M, d->heads, d->batch}, {d->out_row_stride, d->out_head_stride, d->out_batch_stride}};
-    j.res = View4{d->res, {d->N, d->M, d->heads, d->batch}, {d->res_row_stride, d->res_head_stride, d->res_batch_stride}};
-    return run_job(p, j, d->mode, static_cast<cudaStream_t>(stream));
 }

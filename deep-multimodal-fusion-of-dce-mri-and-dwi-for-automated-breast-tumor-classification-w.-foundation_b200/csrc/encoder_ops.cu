@@ -452,44 +452,21 @@ resize_aa_c1_kernel(const float* __restrict__ in, int h, int w, float* __restric
     __stcs(out + (plane * H + oy) * W + ox, acc);
 }
 
-// ------------------------------------------- mask head tail + attention ----
-// MaskHeadResize.out (model_module.py:187, 1x1 Cm->1 + bias) on the `pre` activations, then
-// MaskGuidedSpatialAttention.mask_processor (:67-73, :92-93): 1x1 1->Hc (no bias),
-// GroupNorm(1,Hc), GELU, 1x1 Hc->1 (+bias), sigmoid, clamp to [1e-4, 1-1e-4].
+// ------------------------------------------------------- mask attention ----
+// MaskGuidedSpatialAttention.mask_processor (model_module.py:67-73, :92-93) on a 1-channel mask map:
+// 1x1 1->Hc (no bias), GroupNorm(1,Hc), GELU, 1x1 Hc->1 (+bias), sigmoid, clamp to [1e-4, 1-1e-4].
 // GroupNorm(1,Hc) of u[c,p] = wa[c]*m[p] has mean = mean(wa)*mean(m) and
 // E[u^2] = mean(wa^2)*mean(m^2), so two plane statistics of m suffice.  One CTA per case.
-constexpr int kMaskHidden = 32;
-
-__global__ void mask_tail_kernel(const __nv_bfloat16* __restrict__ pre, int Cm, int npix,
-                                 const float* __restrict__ w_out, const float* __restrict__ b_out,
-                                 float* __restrict__ mask_pred,  // [B, npix]
-                                 int Hc, const float* __restrict__ wa, const float* __restrict__ gn_w,
-                                 const float* __restrict__ gn_b, const float* __restrict__ wb,
-                                 const float* __restrict__ bb, float gn_eps,
-                                 float* __restrict__ attn) {  // [B, npix] or nullptr
+__global__ void mask_attention_kernel(const float* __restrict__ mask, int npix,  // [B, npix]
+                                      int Hc, const float* __restrict__ wa, const float* __restrict__ gn_w,
+                                      const float* __restrict__ gn_b, const float* __restrict__ wb,
+                                      const float* __restrict__ bb, float gn_eps,
+                                      float* __restrict__ attn) {  // [B, npix]
     extern __shared__ float s_m[];  // npix floats
     __shared__ double scratch[33];
     const int b = blockIdx.x;
-    // one thread per pixel: its Cm bf16 activations are one contiguous 2*Cm-byte row (16-byte loads);
-    // with pre == nullptr the mask is already there (emitted by the producing GEMM's fused dot product)
-    for (int p = threadIdx.x; p < npix; p += blockDim.x) {
-        if (pre == nullptr) {
-            s_m[p] = mask_pred[static_cast<size_t>(b) * npix + p];
-            continue;
-        }
-        const uint4* px = reinterpret_cast<const uint4*>(pre + (static_cast<size_t>(b) * npix + p) * Cm);
-        float acc = b_out[0];
-        for (int v = 0; v < Cm / 8; ++v) {
-            float f[8];
-            unpack_bf16x8(__ldg(px + v), f);
-#pragma unroll
-            for (int k = 0; k < 8; ++k) acc = fmaf(f[k], __ldg(w_out + v * 8 + k), acc);
-        }
-        s_m[p] = acc;
-        mask_pred[static_cast<size_t>(b) * npix + p] = acc;
-    }
+    for (int p = threadIdx.x; p < npix; p += blockDim.x) s_m[p] = mask[static_cast<size_t>(b) * npix + p];
     __syncthreads();
-    if (attn == nullptr) return;
     double s1 = 0.0, s2 = 0.0;
     for (int p = threadIdx.x; p < npix; p += blockDim.x) {
         const double m = s_m[p];
@@ -721,20 +698,6 @@ extern "C" int b200_tapsum(const float* d, int B, int H, int W, const float* bia
     return launch_status();
 }
 
-extern "C" int b200_mask_tail(const void* pre, int B, int npix, int Cm, const float* w_out, const float* b_out,
-                              float* mask_pred, int Hc, const float* wa, const float* gn_w, const float* gn_b,
-                              const float* wb, const float* bb, float gn_eps, float* attn, void* stream) {
-    if (B < 0 || npix <= 0 || Cm % 8 != 0 || npix > 12 * 1024) return -1;
-    if (B == 0) return 0;
-    if (pre == nullptr || w_out == nullptr || b_out == nullptr || mask_pred == nullptr) return -2;
-    if (attn != nullptr && (wa == nullptr || gn_w == nullptr || gn_b == nullptr || wb == nullptr || bb == nullptr))
-        return -3;
-    mask_tail_kernel<<<B, 256, npix * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
-        static_cast<const __nv_bfloat16*>(pre), Cm, npix, w_out, b_out, mask_pred, Hc, wa, gn_w, gn_b, wb, bb, gn_eps,
-        attn);
-    return launch_status();
-}
-
 extern "C" int b200_mask_attention(const float* mask, int B, int npix, int Hc, const float* wa, const float* gn_w,
                                    const float* gn_b, const float* wb, const float* bb, float gn_eps, float* attn,
                                    void* stream) {
@@ -743,8 +706,8 @@ extern "C" int b200_mask_attention(const float* mask, int B, int npix, int Hc, c
     if (mask == nullptr || attn == nullptr || wa == nullptr || gn_w == nullptr || gn_b == nullptr || wb == nullptr ||
         bb == nullptr)
         return -2;
-    mask_tail_kernel<<<B, 256, npix * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
-        nullptr, 0, npix, nullptr, nullptr, const_cast<float*>(mask), Hc, wa, gn_w, gn_b, wb, bb, gn_eps, attn);
+    mask_attention_kernel<<<B, 256, npix * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
+        mask, npix, Hc, wa, gn_w, gn_b, wb, bb, gn_eps, attn);
     return launch_status();
 }
 

@@ -1,2 +1,2 @@
 #include "b200_fusion.h"
-extern "C" int b200_abi_version(void) { return 24; }
+extern "C" int b200_abi_version(void) { return 25; }

@@ -15,8 +15,8 @@ here, so this module carries its own feature extractors with timm's parameter na
 RadImageNet) checkpoint's ``state_dict`` loads unchanged - and runs them on the sm_100a kernels:
 
 * ``B200ViTBackbone``: patchify + one GEMM for the patch embedding, an fp32 residual stream, LayerNorm (eps 1e-6),
-  per-head Q.K^T with the softmax numerator fused into the GEMM epilogue (197 keys masked inside a 256-wide tile),
-  P.V with the 1/rowsum applied to the fp32 accumulator, MLP with a fused GELU.
+  one GEMM for qkv, then attention as one ``b200_attention`` launch per block (S = Q K^T per (case, head) in TMEM,
+  the softmax in registers, P V straight off the packed qkv rows), MLP with a fused GELU.
 * ``B200ResNetBackbone``: the 7x7 stem as shared-memory im2col + one GEMM, max-pool, then the 16 bottlenecks as
   implicit GEMMs with folded BatchNorm, ReLU, stride / dilation and the residual in the epilogue.
 

@@ -597,11 +597,10 @@ def _transformer_stage(tr, x, drop=None):
     (DESIGN.md section 2): attn_drop on the softmax probabilities, proj_drop on proj(o) before LayerScale and the
     residual, mlp.drop after the GELU and again on fc2's output before LayerScale and the residual.
 
-    Pre-norm blocks exactly as transformer_model.py:68-133 (eval: dropout is identity); every matmul runs on
-    the tcgen05 GEMM kernel: the patch embedding as a 2x2/stride-2 implicit GEMM, Q.K^T per head with the
-    softmax numerator fused into its epilogue, P.V per head with the 1/rowsum applied to the fp32
-    accumulator (V is produced transposed by putting W_v on the A side; its bias commutes past the
-    row-stochastic P), LayerScale + residual folded into the proj / fc2 epilogues."""
+    Pre-norm blocks exactly as transformer_model.py:68-133 (eval: dropout is identity).  The patch embedding is a
+    2x2/stride-2 implicit GEMM and qkv / proj / fc1 / fc2 run on the tcgen05 GEMM kernel, with LayerScale + residual
+    folded into the proj / fc2 epilogues.  Attention is one b200_attention launch per block: S = Q K^T per
+    (case, head) in TMEM, the softmax in registers, and P V straight off the packed qkv rows."""
     B, H, W, _ = x.shape
     E = tr["E"]
     dev = x.device

@@ -118,42 +118,6 @@ int b200_attention(const void* qkv, int qkv_ld, void* out, int out_ld, int B, in
 int b200_attention_mc(const void* qkv, int qkv_ld, void* out, int out_ld, int B, int N, int heads, int dh, float scale,
                       float drop_p, unsigned long long drop_seed, void* stream);
 
-/*
- * Batched GEMM on the same tcgen05 kernel: for every (batch, head)
- *     out[m, n] = epilogue( sum_k A[m, k] * B[n, k] ),   A, B bf16 K-major, fp32 accumulation.
- * This is how the transformer blocks run (code/transformer_model.py:98-116): Q.K^T per head
- * (mode 1: the epilogue writes exp(alpha*acc - rowmax) as bf16 and 1/rowsum to rowsum_inv - the softmax
- * numerator of :108; columns >= n_valid are masked), P.V^T per head (rowscale = that 1/rowsum, so the
- * division of the softmax is applied to the fp32 accumulator), and V^T = W_v X^T with the weights on the A
- * side (a_shared).  Strides are in elements; rows of A / B must be 16-byte aligned; K tails are zero-filled
- * and ragged M tails clipped by the TMA.  mode 1 needs N == 256 (one tile holds a whole row).
- * scale / bias are indexed n + head * vec_h_stride.
- */
-typedef struct b200_gemm_desc {
-    int M, N, K, heads, batch;
-    const void* a;
-    long long a_row_stride, a_head_stride, a_batch_stride;
-    int a_shared;
-    const void* b;
-    long long b_row_stride, b_head_stride, b_batch_stride;
-    void* out;
-    long long out_row_stride, out_head_stride, out_batch_stride;
-    const void* res;
-    long long res_row_stride, res_head_stride, res_batch_stride;
-    int res_mode, act;
-    const float* scale;
-    const float* bias;
-    int vec_h_stride;
-    const float* rowscale; /* [batch, heads, M] or NULL */
-    int mode;              /* 0 standard, 1 softmax numerator */
-    float alpha;
-    int n_valid;
-    float* rowsum_inv;     /* [batch, heads, M] (mode 1) */
-    int b_rows;            /* valid rows of B per (head, batch); 0 = N.  Rows beyond are read as zeros */
-} b200_gemm_desc;
-
-int b200_gemm_batched(const b200_gemm_desc* d, void* stream);
-
 /* nn.LayerNorm over the last dimension of a token matrix [rows, C] (code/transformer_model.py:16, :71, :73),
  * C a multiple of 256 up to 1024, fp32 statistics; x / y are bf16, or fp32 when x_f32 / y_f32 (the
  * transformer residual stream is kept in fp32). */
@@ -298,11 +262,6 @@ int b200_conv3x3_c1(const void* x, int B, int H, int W, int C, const float* w, c
                     void* stream);
 
 /*
- * MaskHeadResize.out (code/model_module.py:187) on the `pre` activations [B,npix,Cm] bf16
- * -> mask_pred fp32 [B,npix]; when attn != NULL also MaskGuidedSpatialAttention's
- * mask_processor (:67-73, :92-93) -> attention map fp32 [B,npix] in [1e-4, 1-1e-4].
- */
-/*
  * MaskGuidedSpatialAttention.mask_processor (code/model_module.py:67-73, :92-93) on an fp32 1-channel map
  * mask [B,npix] -> attention map fp32 [B,npix] clamped to [1e-4, 1-1e-4].
  */
@@ -319,10 +278,6 @@ int b200_resize_bilinear_c1(const float* in, int B, int h, int w, float* out, in
  * than `input_size`; code/parameters_generate.py:68).  ATen's separable triangle filter of support max(in/out, 1),
  * horizontal pass then vertical, fp32.  Growing sides reduce to the plain bilinear taps. */
 int b200_resize_aa_c1(const float* in, int B, int h, int w, float* out, int H, int W, void* stream);
-
-int b200_mask_tail(const void* pre, int B, int npix, int Cm, const float* w_out, const float* b_out,
-                   float* mask_pred, int Hc, const float* wa, const float* gn_w, const float* gn_b, const float* wb,
-                   const float* bb, float gn_eps, float* attn, void* stream);
 
 /* First Projector layer on a 1-channel map (code/model_module.py:338-340, :639-640). */
 int b200_lift_c1(const float* r, long long total_pix, int N, const float* w, const float* scale, const float* bias,

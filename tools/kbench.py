@@ -19,7 +19,7 @@ DEV = "cuda"
 
 
 def conv_case(name, B, H, W, cin, cout, taps, res_mode=0, act=1, gap=False, n_split=None, up2=False, dot=False,
-              store=True):
+              store=True, drop=False):
     x = (torch.randn(B, H, W, cin, device=DEV) * 0.5).bfloat16()
     w = (torch.randn(cout, taps * cin, device=DEV) / math.sqrt(taps * cin)).bfloat16()
     scale = torch.rand(cout, device=DEV) + 0.5
@@ -34,13 +34,29 @@ def conv_case(name, B, H, W, cin, cout, taps, res_mode=0, act=1, gap=False, n_sp
 
     def run():
         nat.conv_gemm(x, w, taps=taps, scale=scale, bias=bias, res=res, res_mode=res_mode, act=act, out=out, up2=up2,
-                      gap=gapb, n_split=n_split, act2=1, out2=out2, dot_w=dw, dot_out=dout, store=store)
+                      gap=gapb, n_split=n_split, act2=1, out2=out2, dot_w=dw, dot_out=dout, store=store,
+                      dropout=(0.1, 7, 1) if drop else None)
 
     px = B * H * W
     byts = px * cin * 2 + (px * n1 * 2 * (4 if up2 else 1) if store else 0) + (px * (cout - n1) * 2 if n_split else 0) \
         + (px * n1 * 2 if res_mode else 0) + (px * 36 if dot else 0) + cout * taps * cin * 2
     flops = 2.0 * px * cout * taps * cin
     return name, run, byts, flops
+
+
+def linear_mc_case(name, M, K, N):
+    """Transformer proj / fc2 under MC dropout: fp32 residual stream, out = res + drop(x w^T * scale + bias)."""
+    x = (torch.randn(M, K, device=DEV) * 0.5).bfloat16()
+    w = (torch.randn(N, K, device=DEV) / math.sqrt(K)).bfloat16()
+    scale = torch.rand(N, device=DEV) + 0.5
+    bias = torch.randn(N, device=DEV) * 0.1
+    res = torch.randn(M, N, device=DEV)
+    out = torch.empty(M, N, device=DEV)
+
+    def run():
+        nat.linear_f32(x, w, scale=scale, bias=bias, res=res, res_mode=2, out=out, dropout=(0.1, 7))
+
+    return name, run, M * K * 2 + M * N * 8 + N * K * 2, 2.0 * M * N * K
 
 
 def vit_bench(batch, iters):
@@ -102,6 +118,10 @@ def main():
         conv_case("1x1 128->64 gelu (proj)", B, 32, 32, 128, 64, 1),
         conv_case("1x1 64->64 gelu up2 (proj out)", B, 32, 32, 64, 64, 1, up2=True),
         conv_case("1x1 64->64 gelu", B, 32, 32, 64, 64, 1),
+        conv_case("1x1 128->128 gelu mc-dropout", B, 32, 32, 128, 128, 1, drop=True),
+        conv_case("1x1 128->64 gelu mc-dropout", B, 32, 32, 128, 64, 1, drop=True),
+        linear_mc_case("linear 2048->512 fp32 res mc-dropout (fc2)", B * 256, 2048, 512),
+        linear_mc_case("linear 512->128 fp32 res mc-dropout", B * 256, 512, 128),
     ]
     import numpy as np
     import dataset as b_dataset
